@@ -2,6 +2,7 @@
 """bench.py - audio samples/sec of the Harmonic(100)+FilteredNoise(65) decoder.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+                  [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N \
       --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
@@ -132,6 +133,24 @@ class ClockSampler:
     return {'sm_mhz': statistics.median(r[1] for r in rows),
             'sm_max_mhz': self.smax, 'samples': len(rows), 'window': window,
             'reasons': reasons}
+
+
+DUMP_ITEMS = 64   # batch items --dump-outputs keeps (64 x 64000 float32 audio = 16 MB)
+
+
+def dump_outputs(path, arrays):
+  """Writes `arrays` (name -> tensor, batch first) as path/<name>.npy in float32.
+  Outputs with more than DUMP_ITEMS batch items keep a fixed, seeded choice of
+  DUMP_ITEMS of them, the same items in every run, so that two builds can be
+  compared output for output."""
+  import torch
+  os.makedirs(path, exist_ok=True)
+  for name, t in arrays.items():
+    x = t.detach()
+    if x.dim() and x.shape[0] > DUMP_ITEMS:
+      idx = np.sort(np.random.default_rng(0).choice(x.shape[0], DUMP_ITEMS, replace=False))
+      x = x[torch.from_numpy(idx).to(x.device)]
+    np.save(os.path.join(path, name + '.npy'), x.float().cpu().numpy())
 
 
 def make_host_inputs(batch, seed):
@@ -370,12 +389,13 @@ def run_ours(args):
       graph_note = 'eager ProcessorGroup.__call__ (graph capture failed: %r)' % (e,)
       torch.cuda.synchronize()
 
+  eager_out = {}
   if graphs:
     def step_resident(i):
       graphs[i % n_sets].replay()
   else:
     def step_resident(i):
-      group(dev_sets[i % n_sets])
+      eager_out['audio'] = group(dev_sets[i % n_sets])
 
   sampler = ClockSampler(local_rank)
   if rank == 0:
@@ -390,6 +410,10 @@ def run_ours(args):
     launches_timed = launches * args.steps // (args.steps + args.warmup)
   ms_per_step = ms_total / args.steps
   value = world * B * N_SAMPLES / (ms_per_step * 1e-3)
+  if args.dump_outputs and rank == 0:
+    # the audio of the last timed step (rank 0's shard when sharded)
+    dump_outputs(args.dump_outputs, {'audio': graph_out[
+        (args.warmup + args.steps - 1) % n_sets] if graphs else eager_out['audio']})
 
   # -- e2e: host buffers in, host audio out, copies inside the timed region ---
   # The public host-buffer call: HostDecoder = ProcessorGroup over pinned host
@@ -812,6 +836,12 @@ def run_c4(args):
   sampler.mark_timed(0)
   ms_step = timed(step, args.steps, args.warmup) / args.steps
   sampler.mark_timed(1)
+  if args.dump_outputs and rank == 0:
+    # loss and input gradients of the last timed step (before the graph capture
+    # below overwrites the gradients)
+    d = sets[(args.warmup + args.steps - 1) % len(sets)]
+    dump_outputs(args.dump_outputs, dict(
+        loss=last['loss'], **{'grad_' + k: d[k].grad for k in grad_keys}))
   launches = (lib.ddsp_b200_launch_count() - c0) * args.steps // (args.steps + args.warmup)
   value = world * B * N_SAMPLES / (ms_step * 1e-3)
 
@@ -961,7 +991,8 @@ def main():
 def _main():
   ap = argparse.ArgumentParser()
   ap.add_argument('--gpus', type=int, default=1)
-  ap.add_argument('--steps', type=int, default=50)
+  ap.add_argument('--steps', type=int, default=None,
+                  help='timed steps (default 50; 10 with --config c4)')
   ap.add_argument('--warmup', type=int, default=10)
   ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
   ap.add_argument('--batch', type=int, default=BATCH_PER_GPU,
@@ -976,11 +1007,18 @@ def _main():
   ap.add_argument('--config', default='decoder', choices=['decoder', 'c4'],
                   help="'decoder' (default): configs[2] / configs[4]; 'c4': configs[3], "
                        'forward + backward through SpectralLoss, batch 128 per GPU')
+  ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                  help='after the timed steps, write what the last one computed as '
+                       'DIR/<name>.npy (decoder: audio; c4: loss and input gradients)')
   args = ap.parse_args()
+  if args.steps is None:
+    args.steps = 10 if args.config == 'c4' else 50
+  if args.steps < 1:
+    ap.error('--steps must be at least 1')
+  if args.dump_outputs and args.impl != 'ours':
+    ap.error('--dump-outputs writes the outputs of --impl ours')
   args.warmup = max(args.warmup, 3)
   if args.config == 'c4':
-    if args.steps == 50:
-      args.steps = 10
     return run_c4_reference(args) if args.impl == 'reference' else run_c4(args)
   if args.impl == 'reference':
     return run_reference(args)

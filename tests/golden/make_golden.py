@@ -14,11 +14,13 @@ Needs /root/reference, so it runs in the authoring container only:
   python tests/golden/make_golden.py          # rewrite every fixture
   python tests/golden/make_golden.py --check  # regenerate in memory and compare
 
-The fixtures travel to the GPU box; tests/test_reference_pin.py (CPU: oracle vs
-fixtures, and fixtures vs a fresh reference run when the reference is present)
-and tests/test_gpu_golden.py (CUDA path vs fixtures) read them.  Inputs are
-regenerated from their seeds by tests/util.synth_inputs; an input checksum in
-every fixture guards against generator drift.
+The tests read the fixtures, so they need no reference: tests/test_reference_pin.py
+(CPU: oracle vs fixtures, and fixtures vs a fresh reference run when the reference
+is present), tests/test_gpu_golden.py (CUDA path vs fixtures), and
+tests/test_reference_fuzz.py, test_effects.py and test_host_api.py (oracle and host
+logic vs the reference on the argument sets drawn by the *_cases generators below).
+Inputs are regenerated from their seeds by tests/util.synth_inputs; an input
+checksum in every fixture guards against generator drift.
 """
 import os
 import sys
@@ -243,15 +245,289 @@ def impulse_responses():
   return out
 
 
+SAMPLE = 512
+
+
+def sample_index(size):
+  """Flat indices of the stored part of an output of `size` elements: all of them
+  up to SAMPLE, else a fixed seeded choice of SAMPLE."""
+  if size <= SAMPLE:
+    return np.arange(size)
+  return np.sort(np.random.default_rng(size).choice(size, SAMPLE, replace=False))
+
+
+def pack_outputs(outputs):
+  """{name: array, or None where the reference raised} -> fixture entries: for
+  each output its shape, its sample_index values, and its peak and L2 norm over
+  every element, in a few flat arrays (one small array per output would make the
+  file mostly zip headers)."""
+  names, ndim, dims, start, values, absmax, l2 = [], [], [], [0], [], [], []
+  for name, x in outputs.items():
+    names.append(name)
+    x = None if x is None else np.asarray(x, np.float64)
+    ndim.append(-1 if x is None else x.ndim)
+    dims.append(([] if x is None else list(x.shape)) + [0] * (4 - (0 if x is None else x.ndim)))
+    v = np.zeros(0) if x is None else x.ravel()[sample_index(x.size)]
+    values.append(v)
+    start.append(start[-1] + v.size)
+    absmax.append(np.abs(x).max() if x is not None and x.size else 0.0)
+    l2.append(0.0 if x is None else np.sqrt((x * x).sum()))
+  return dict(names=np.array(names), ndim=np.array(ndim, np.int64),
+              dims=np.array(dims, np.int64), start=np.array(start, np.int64),
+              values=np.concatenate(values), absmax=np.array(absmax),
+              l2=np.array(l2))
+
+
+def unpack_outputs(g):
+  """pack_outputs entries -> {name: None where the reference raised, else
+  (shape, sampled values, peak, L2 norm)}."""
+  out = {}
+  for i, name in enumerate(g['names']):
+    n = int(g['ndim'][i])
+    out[str(name)] = None if n < 0 else (
+        tuple(int(d) for d in g['dims'][i][:n]),
+        g['values'][g['start'][i]:g['start'][i + 1]], float(g['absmax'][i]),
+        float(g['l2'][i]))
+  return out
+
+
+def fuzz_fft_convolve_cases():
+  """Arguments of core.fft_convolve: shapes, both paddings, delay compensations."""
+  rng = np.random.default_rng(123)
+  for _ in range(24):
+    b, f = int(rng.integers(1, 3)), int(rng.choice([1, 2, 5, 10, 25]))
+    frame, s = int(rng.choice([1, 3, 16, 48, 64])), int(rng.choice([1, 2, 3, 10, 31, 64, 65, 128, 200]))
+    pad, dc = str(rng.choice(['same', 'valid'])), int(rng.choice([-1, 0, 1, 5]))
+    a = rng.standard_normal((b, f * frame)).astype(np.float32)
+    ir = rng.standard_normal((b, f, s)).astype(np.float32)
+    yield dict(a=a, ir=ir, padding=pad, delay_compensation=dc)
+
+
+def fuzz_frequency_filter_cases():
+  """core.frequency_filter with odd / even / degenerate windows."""
+  rng = np.random.default_rng(124)
+  for _ in range(20):
+    f, frame = int(rng.choice([1, 4, 10])), int(rng.choice([8, 32, 64]))
+    nb = int(rng.choice([2, 3, 9, 16, 33, 65, 100, 129, 130, 257]))
+    ws = int(rng.choice([0, 1, 2, 3, 7, 8, 50, 51, 64, 65, 257]))
+    a = rng.uniform(-1, 1, (1, f * frame)).astype(np.float32)
+    m = rng.uniform(0, 1, (1, f, nb)).astype(np.float32)
+    yield dict(audio=a, magnitudes=m, window_size=ws)
+
+
+def fuzz_harmonic_synthesis_cases():
+  """core.harmonic_synthesis over every amplitude resampling method, both phase
+  accumulators, sample rates and the optional arguments."""
+  rng = np.random.default_rng(321)
+  for _ in range(14):
+    b, f = int(rng.integers(1, 3)), int(rng.choice([2, 5, 10, 25]))
+    hop, k = int(rng.choice([4, 16, 64, 100])), int(rng.choice([1, 3, 20, 60]))
+    method = str(rng.choice(['window', 'linear', 'nearest', 'cubic']))
+    uac, sr = bool(rng.integers(0, 2)), int(rng.choice([16000, 8000, 44100]))
+    f0 = rng.uniform(20, sr * 0.45, (b, f, 1)).astype(np.float32)
+    amp = rng.uniform(0, 1, (b, f, 1)).astype(np.float32)
+    hd = rng.uniform(0, 1, (b, f, k)).astype(np.float32) if rng.integers(0, 4) else None
+    shifts = (rng.uniform(-0.05, 0.05, (b, f, k)).astype(np.float32)
+              if hd is not None and rng.integers(0, 2) else None)
+    yield dict(f0=f0, amp=amp, hd=hd, shifts=shifts, n_samples=f * hop, sample_rate=sr,
+               method=method, use_angular_cumsum=uac)
+
+
+def fuzz_misc_cases():
+  """(kind, arguments) for Harmonic.get_controls, oscillator_bank, streaming
+  synthesis, the scaling functions and Sinusoidal, drawn from one generator."""
+  rng = np.random.default_rng(999)
+  for _ in range(8):                                   # Harmonic.get_controls variants
+    f, k = int(rng.choice([3, 10])), int(rng.choice([1, 7, 40]))
+    scale, nyq, sr = bool(rng.integers(0, 2)), bool(rng.integers(0, 2)), int(rng.choice([16000, 4000]))
+    a = rng.standard_normal((1, f, 1)).astype(np.float32)
+    h = rng.standard_normal((1, f, k)).astype(np.float32)
+    f0 = rng.uniform(0, sr / 2, (1, f, 1)).astype(np.float32)
+    if not scale:
+      a, h = np.abs(a), np.abs(h)
+    yield 'get_controls', dict(a=a, h=h, f0=f0, f=f, scale=scale, nyquist=nyq, sample_rate=sr)
+  for _ in range(8):                                   # oscillator_bank
+    b, n, k = int(rng.integers(1, 3)), int(rng.choice([50, 1000, 2500])), int(rng.choice([1, 4, 17]))
+    sr, ss, uac = int(rng.choice([16000, 8000])), bool(rng.integers(0, 2)), bool(rng.integers(0, 2))
+    fe = rng.uniform(0, sr * 0.6, (b, n, k)).astype(np.float32)
+    ae = rng.uniform(0, 1, (b, n, k)).astype(np.float32)
+    yield 'oscillator_bank', dict(fe=fe, ae=ae, sample_rate=sr, sum_sinusoids=ss,
+                                  use_angular_cumsum=uac)
+  for _ in range(8):                                   # streaming synthesis, carried phase
+    b, f, hop = int(rng.integers(1, 3)), int(rng.choice([1, 4, 10])), int(rng.choice([16, 64]))
+    k = int(rng.choice([1, 5, 30]))
+    f0 = rng.uniform(50, 2000, (b, f, 1)).astype(np.float32)
+    amp = rng.uniform(0, 1, (b, f, 1)).astype(np.float32)
+    hd = rng.uniform(0, 1, (b, f, k)).astype(np.float32) if rng.integers(0, 3) else None
+    ph = rng.uniform(0, 6.28, (b, 1, 1)).astype(np.float32) if rng.integers(0, 2) else None
+    method = str(rng.choice(['linear', 'window']))
+    yield 'streaming', dict(f0=f0, amp=amp, hd=hd, phase=ph, n_samples=f * hop,
+                            method=method)
+  for _ in range(5):                                   # scaling functions
+    x = (4 * rng.standard_normal((2, 5, 7))).astype(np.float32)
+    ex, mv, th = float(rng.choice([10.0, 2.0, 5.0])), float(rng.choice([2.0, 1.0])), float(rng.choice([1e-7, 1e-3]))
+    depth = int(rng.choice([1, 8, 64]))
+    fr = rng.standard_normal((2, 5, 3 * depth)).astype(np.float32)
+    yield 'scalers', dict(x=x, exponent=ex, max_value=mv, threshold=th, fr=fr, depth=depth)
+  for _ in range(4):                                   # Sinusoidal
+    f, k, hop = int(rng.choice([5, 10])), int(rng.choice([1, 4, 9])), int(rng.choice([16, 64]))
+    a = rng.standard_normal((1, f, k)).astype(np.float32)
+    fr = rng.standard_normal((1, f, k)).astype(np.float32)
+    method = str(rng.choice(['window', 'linear']))
+    yield 'sinusoidal', dict(a=a, fr=fr, n_samples=f * hop, method=method)
+
+
+def reference_fuzz():
+  """The reference in its wide mode (its own code evaluated in float64) on the
+  fuzz_*_cases arguments: what tests/test_reference_fuzz.py holds the oracle's
+  float64 mode to, packed by pack_outputs under the names
+  <function>_<case>[_<output>]."""
+  ddsp = ref_on_shim.load()
+  tf = ref_on_shim.tf()
+  t = tf.convert_to_tensor
+  tt = lambda x: None if x is None else t(x)  # noqa: E731
+
+  def wide(fn):
+    tf.set_wide(True)
+    try:
+      return ref_on_shim.to_numpy(fn())
+    finally:
+      tf.set_wide(False)
+
+  out = {}
+  for i, c in enumerate(fuzz_fft_convolve_cases()):
+    try:
+      want = wide(lambda: ddsp.core.fft_convolve(c['a'], c['ir'], padding=c['padding'],
+                                                 delay_compensation=c['delay_compensation']))
+    except Exception:  # pylint: disable=broad-except
+      want = None
+    out['fft_convolve_%d' % i] = want
+  for i, c in enumerate(fuzz_frequency_filter_cases()):
+    out['frequency_filter_%d' % i] = wide(lambda: ddsp.core.frequency_filter(
+        c['audio'], c['magnitudes'], window_size=c['window_size']))
+  for i, c in enumerate(fuzz_harmonic_synthesis_cases()):
+    # tensors, so that the wide mode widens every operand (a raw float32 array in
+    # `1.0 + harmonic_shifts` would be rounded by NumPy before the shim sees it)
+    out['harmonic_synthesis_%d' % i] = wide(lambda: ddsp.core.harmonic_synthesis(
+        t(c['f0']), t(c['amp']), harmonic_shifts=tt(c['shifts']),
+        harmonic_distribution=tt(c['hd']), n_samples=c['n_samples'],
+        sample_rate=c['sample_rate'], amp_resample_method=c['method'],
+        use_angular_cumsum=c['use_angular_cumsum']))
+  for i, (kind, c) in enumerate(fuzz_misc_cases()):
+    key = '%s_%d' % (kind, i)
+    if kind == 'get_controls':
+      syn = ddsp.synths.Harmonic(n_samples=c['f'] * 8, sample_rate=c['sample_rate'],
+                                 scale_fn=ddsp.core.exp_sigmoid if c['scale'] else None,
+                                 normalize_below_nyquist=c['nyquist'])
+      want = wide(lambda: syn.get_controls(c['a'], c['h'], c['f0']))
+      for name in ('amplitudes', 'harmonic_distribution', 'f0_hz'):
+        out['%s_%s' % (key, name)] = want[name]
+    elif kind == 'oscillator_bank':
+      out[key] = wide(lambda: ddsp.core.oscillator_bank(
+          t(c['fe']), t(c['ae']), sample_rate=c['sample_rate'],
+          sum_sinusoids=c['sum_sinusoids'], use_angular_cumsum=c['use_angular_cumsum']))
+    elif kind == 'streaming':
+      audio, phase = wide(lambda: list(ddsp.core.streaming_harmonic_synthesis(
+          t(c['f0']), t(c['amp']), tt(c['hd']), tt(c['phase']), n_samples=c['n_samples'],
+          sample_rate=16000, amp_resample_method=c['method'])))
+      out[key + '_audio'], out[key + '_phase'] = audio, phase
+    elif kind == 'scalers':
+      out[key + '_exp_sigmoid'] = wide(lambda: ddsp.core.exp_sigmoid(
+          t(c['x']), c['exponent'], c['max_value'], c['threshold']))
+      out[key + '_sigmoid'] = wide(lambda: ddsp.core.frequencies_sigmoid(
+          t(c['fr']), depth=c['depth']))
+      out[key + '_softmax'] = wide(lambda: ddsp.core.frequencies_softmax(
+          t(c['fr']), depth=c['depth']))
+    else:
+      syn = ddsp.synths.Sinusoidal(n_samples=c['n_samples'], sample_rate=16000,
+                                   amp_resample_method=c['method'])
+      out[key] = wide(lambda: syn(t(c['a']), t(c['fr'])))
+  return pack_outputs(out)
+
+
+WINDOW_CASES = [(128, 0, False), (128, 257, False), (128, 64, False), (128, 63, False),
+                (30, 257, False), (2048, 257, True), (100, 51, True), (100, 50, False),
+                (4, 0, False)]
+CROP_CASES = [(64192, 64000, 128, 'same', -1), (64192, 64000, 128, 'valid', -1),
+              (1009, 1000, 10, 'same', 0), (109, 10, 100, 'same', -1),
+              (4095, 1000, 3000, 'same', 0), (3999, 1000, 3000, 'valid', -1)]
+
+
+def host_helper_cases():
+  """(kind, arguments) for core.apply_window_to_impulse_response and
+  core.crop_and_compensate_delay."""
+  rng = np.random.default_rng(0)
+  for ir_size, ws, causal in WINDOW_CASES:
+    ir = rng.standard_normal((2, 3, ir_size)).astype(np.float32)
+    yield 'window', (ir, ws, causal)
+  for total, n, s, pad, dc in CROP_CASES:
+    a = rng.standard_normal((2, total)).astype(np.float32)
+    yield 'crop', (a, n, s, pad, dc)
+
+
+def host_helpers():
+  """The reference's float32 results on host_helper_cases, for
+  tests/test_host_api.py."""
+  ddsp = ref_on_shim.load()
+  out = {}
+  for i, (kind, args) in enumerate(host_helper_cases()):
+    fn = (ddsp.core.apply_window_to_impulse_response if kind == 'window' else
+          ddsp.core.crop_and_compensate_delay)
+    out['%s_%d' % (kind, i)] = ref_on_shim.to_numpy(fn(*args))
+  return pack_outputs(out)
+
+
+def filtered_noise_reverb_case(trainable):
+  """Shapes and draws of the FilteredNoiseReverb composition check: audio, the
+  magnitudes (one learned set when trainable) and the noise the synthesizer uses."""
+  rng = np.random.default_rng(5)
+  B, N, L, F, NB, WS = 2, 3000, 1920, 40, 16, 257
+  audio = rng.standard_normal((B, N)).astype(np.float32)
+  mags = rng.standard_normal((1 if trainable else B, F, NB)).astype(np.float32)
+  noise = rng.uniform(-1, 1, (mags.shape[0], L)).astype(np.float32)
+  kw = dict(trainable=trainable, reverb_length=L, window_size=WS, n_frames=F,
+            n_filter_banks=NB)
+  return audio, mags, noise, kw
+
+
+def filtered_noise_reverb():
+  """effects.FilteredNoiseReverb (the reference's class, float32) on
+  filtered_noise_reverb_case, with its tf.random.uniform draw pinned to the case's
+  noise, fixed and trainable: for tests/test_effects.py."""
+  ddsp = ref_on_shim.load()
+  tf = ref_on_shim.tf()
+  out = {}
+  for trainable in (False, True):
+    audio, mags, noise, kw = filtered_noise_reverb_case(trainable)
+    uniform = tf.random.uniform
+    tf.random.uniform = lambda shape, minval=0, maxval=1, **_: tf.constant(noise)
+    try:
+      r = ddsp.effects.FilteredNoiseReverb(**kw)
+      if trainable:
+        r.build(None)
+        r._magnitudes = tf.constant(mags[0])
+        want = ref_on_shim.to_numpy(r(audio))
+      else:
+        want = ref_on_shim.to_numpy(r(audio, mags))
+    finally:
+      tf.random.uniform = uniform
+    out['audio_trainable_%d' % trainable] = want
+  return out
+
+
 FIXTURES = dict(c1_harmonic=c1_harmonic, decoder_small=decoder_small, c2_item=c2_item,
                 harmonic_shifts=harmonic_shifts, resample_methods=resample_methods,
                 angular_cumsum=angular_cumsum, spectral_loss=spectral_loss,
-                impulse_responses=impulse_responses)
+                impulse_responses=impulse_responses, reference_fuzz=reference_fuzz,
+                host_helpers=host_helpers, filtered_noise_reverb=filtered_noise_reverb)
 
 
 def compare(name, got, want, atol=0.0):
   assert set(want.files) == set(got), (name, sorted(set(want.files) ^ set(got)))
   for k in want.files:
+    if want[k].dtype.kind == 'U':
+      np.testing.assert_array_equal(got[k], want[k], err_msg='%s/%s' % (name, k))
+      continue
     np.testing.assert_allclose(np.asarray(got[k], np.float64),
                                np.asarray(want[k], np.float64), rtol=0, atol=atol,
                                err_msg='%s/%s' % (name, k))

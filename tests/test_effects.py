@@ -4,6 +4,8 @@ core.fft_convolve (framed FFT convolution on torch.fft / cuFFT).
 CPU: the FFT formulation against the oracle's literal restatement of
 core.py:1382-1473, for single-frame (reverb) and multi-frame IRs.  GPU: the
 processors against the float64 oracle through both routes of fft_convolve."""
+import os
+
 import numpy as np
 import pytest
 import torch
@@ -67,35 +69,19 @@ def test_filtered_noise_reverb_constructor_and_errors():
 @pytest.mark.parametrize('trainable', [False, True])
 def test_filtered_noise_reverb_composition_matches_reference(monkeypatch, trainable):
   """The host logic of FilteredNoiseReverb (effects.py:202-278 on top of Reverb's
-  28-117) against the UNMODIFIED reference class run on the NumPy shim, with the
-  same noise and, when trainable, the same learned magnitudes.  The CUDA kernels
-  are replaced by the oracle here (they have their own parity tests): what is under
-  test is the composition - scale + bias, synthesis of the impulse response, tiling
-  of the single learned response, dry-tap masking, 'same' convolution with zero
-  delay compensation, dry mix."""
-  from oracle import ref_on_shim
-  if not ref_on_shim.available():
-    pytest.skip('reference sources not present')
+  28-117) against the UNMODIFIED reference class, with the same noise and, when
+  trainable, the same learned magnitudes (tests/golden/filtered_noise_reverb.npz,
+  made by make_golden.py on the NumPy shim).  The CUDA kernels are replaced by the
+  oracle here (they have their own parity tests): what is under test is the
+  composition - scale + bias, synthesis of the impulse response, tiling of the
+  single learned response, dry-tap masking, 'same' convolution with zero delay
+  compensation, dry mix."""
   from ddsp_b200 import effects
-  ref = ref_on_shim.load()
-  tf = ref_on_shim.tf()
-  rng = np.random.default_rng(5)
-  B, N, L, F, NB, WS = 2, 3000, 1920, 40, 16, 257
-  audio = rng.standard_normal((B, N)).astype(np.float32)
-  mags = rng.standard_normal((1 if trainable else B, F, NB)).astype(np.float32)
-  noise = rng.uniform(-1, 1, (mags.shape[0], L)).astype(np.float32)
-
-  # ---- the reference, on the shim, with its random draw pinned ----
-  monkeypatch.setattr(tf.random, 'uniform',
-                      lambda shape, minval=0, maxval=1, **kw: tf.constant(noise))
-  r = ref.effects.FilteredNoiseReverb(trainable=trainable, reverb_length=L, window_size=WS,
-                                      n_frames=F, n_filter_banks=NB)
-  if trainable:
-    r.build(None)
-    r._magnitudes = tf.constant(mags[0])
-    want = ref_on_shim.to_numpy(r(audio))
-  else:
-    want = ref_on_shim.to_numpy(r(audio, mags))
+  from tests.golden import make_golden as mg
+  audio, mags, noise, reverb_kw = mg.filtered_noise_reverb_case(trainable)
+  B, N = audio.shape
+  want = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden',
+                              'filtered_noise_reverb.npz'))['audio_trainable_%d' % trainable]
 
   # ---- ours, kernels swapped for the oracle ----
   def t32(x, device=None):
@@ -114,8 +100,7 @@ def test_filtered_noise_reverb_composition_matches_reference(monkeypatch, traina
                           o.fft_convolve(t32(a).numpy(), t32(ir).numpy(), padding=padding,
                                          delay_compensation=delay_compensation,
                                          dtype=np.float32)))
-  rev = effects.FilteredNoiseReverb(trainable=trainable, reverb_length=L, window_size=WS,
-                                    n_frames=F, n_filter_banks=NB)
+  rev = effects.FilteredNoiseReverb(**reverb_kw)
   rev._synth.injected_noise = torch.from_numpy(noise)
   with torch.no_grad():
     if trainable:

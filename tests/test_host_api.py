@@ -299,34 +299,35 @@ def test_host_decoder_rejects_non_decoder_dags():
 def test_window_and_crop_helpers_match_oracle_and_reference():
   """core.apply_window_to_impulse_response (core.py:1477-1531) and
   core.crop_and_compensate_delay (1338-1379): host-side torch ops, so they run on
-  the CPU - against the oracle everywhere and the unmodified reference where present."""
+  the CPU - against the oracle and the unmodified reference's results
+  (tests/golden/host_helpers.npz: shape, peak and L2 norm of each output and up to
+  make_golden.SAMPLE of its elements)."""
   import torch
   from oracle import ddsp_oracle as o
-  from oracle import ref_on_shim
-  ref = ref_on_shim.load() if ref_on_shim.available() else None
-  rng = np.random.default_rng(0)
-  for ir_size, ws, causal in [(128, 0, False), (128, 257, False), (128, 64, False),
-                              (128, 63, False), (30, 257, False), (2048, 257, True),
-                              (100, 51, True), (100, 50, False), (4, 0, False)]:
-    ir = rng.standard_normal((2, 3, ir_size)).astype(np.float32)
-    got = core.apply_window_to_impulse_response(ir, ws, causal)
-    assert isinstance(got, torch.Tensor) and not got.is_cuda
-    want = o.apply_window_to_impulse_response(ir, ws, causal, dtype=np.float32)
-    assert tuple(got.shape) == want.shape
-    assert np.abs(got.numpy() - want).max() < 1e-6
-    if ref is not None:
-      want = ref_on_shim.to_numpy(ref.core.apply_window_to_impulse_response(ir, ws, causal))
+  from tests.golden import make_golden as mg
+  ref = mg.unpack_outputs(np.load(os.path.join(ROOT, 'tests', 'golden', 'host_helpers.npz')))
+  for i, (kind, args) in enumerate(mg.host_helper_cases()):
+    shape, values, peak, l2 = ref['%s_%d' % (kind, i)]
+    if kind == 'window':
+      ir, ws, causal = args
+      got = core.apply_window_to_impulse_response(ir, ws, causal)
+      assert isinstance(got, torch.Tensor) and not got.is_cuda
+      want = o.apply_window_to_impulse_response(ir, ws, causal, dtype=np.float32)
+      assert tuple(got.shape) == want.shape
       assert np.abs(got.numpy() - want).max() < 1e-6
-  for total, n, s, pad, dc in [(64192, 64000, 128, 'same', -1), (64192, 64000, 128, 'valid', -1),
-                               (1009, 1000, 10, 'same', 0), (109, 10, 100, 'same', -1),
-                               (4095, 1000, 3000, 'same', 0), (3999, 1000, 3000, 'valid', -1)]:
-    a = rng.standard_normal((2, total)).astype(np.float32)
-    got = core.crop_and_compensate_delay(a, n, s, pad, dc).numpy()
-    want = o.crop_and_compensate_delay(a, n, s, pad, dc)
-    assert np.array_equal(got, want)
-    if ref is not None:
-      assert np.array_equal(got, ref_on_shim.to_numpy(
-          ref.core.crop_and_compensate_delay(a, n, s, pad, dc)))
+      got = got.numpy().astype(np.float64)
+      assert got.shape == shape, (args[1:], got.shape, shape)
+      assert np.abs(got.ravel()[mg.sample_index(got.size)] - values).max() < 1e-6
+      assert abs(np.abs(got).max() - peak) < 1e-6
+      assert abs(np.sqrt((got * got).sum()) - l2) < 1e-6 * np.sqrt(got.size)
+    else:
+      got = core.crop_and_compensate_delay(*args).numpy()
+      assert np.array_equal(got, o.crop_and_compensate_delay(*args))
+      got = got.astype(np.float64)
+      assert got.shape == shape, (args[1:], got.shape, shape)
+      assert np.array_equal(got.ravel()[mg.sample_index(got.size)], values)
+      assert (np.abs(got).max() if got.size else 0.0) == peak
+      assert abs(np.sqrt((got * got).sum()) - l2) <= 1e-12 * l2   # summation order only
   with pytest.raises(ValueError, match="Padding must be 'valid' or 'same'"):
     core.crop_and_compensate_delay(np.zeros((1, 10), np.float32), 5, 3, 'full', 0)
 

@@ -1,178 +1,119 @@
-"""Randomised cross-check of the oracle against the UNMODIFIED reference run on the
-NumPy shim (CPU, authoring container only: skipped where /root/reference is absent).
+"""Randomised cross-check of the oracle against the UNMODIFIED reference (CPU).
 
 The golden fixtures pin the oracle on the path's configurations; this sweeps the
 argument space around them - shapes, paddings, delays, odd / even / degenerate filter
 windows, every amplitude resampling method, both phase accumulators, sample rates,
 optional arguments - in the reference's "wide" mode (its own code evaluated in float64)
 against the oracle's float64 mode.  It is how the odd-window Hann discrepancy was found.
+
+The arguments are drawn from fixed seeds by the fuzz_*_cases generators of
+tests/golden/make_golden.py; the reference's results on them are in
+tests/golden/reference_fuzz.npz (each output's shape, peak and L2 norm, and up to
+make_golden.SAMPLE of its elements), and test_reference_pin.py checks that file
+against a fresh reference run wherever the reference sources are present.
 """
+import os
+
 import numpy as np
 import pytest
 
 from oracle import ddsp_oracle as o
-from oracle import ref_on_shim
+from tests.golden import make_golden as mg
 
-pytestmark = pytest.mark.skipif(
-    not ref_on_shim.available(),
-    reason='reference sources (/root/reference) are only in the authoring container')
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
 
 
 @pytest.fixture(scope='module')
 def ref():
-  return ref_on_shim.load(), ref_on_shim.tf()
-
-
-def _wide(tf, fn):
-  tf.set_wide(True)
-  try:
-    return ref_on_shim.to_numpy(fn())
-  finally:
-    tf.set_wide(False)
+  return mg.unpack_outputs(np.load(os.path.join(GOLD, 'reference_fuzz.npz')))
 
 
 def _close(got, want, tol, what):
-  got, want = np.asarray(got, np.float64), np.asarray(want, np.float64)
-  assert got.shape == want.shape, (what, got.shape, want.shape)
+  """The whole of `got` against a stored reference output: same shape, the stored
+  elements within tol * max(1, peak), and peak and L2 norm within what that
+  elementwise bound allows."""
+  shape, values, peak, l2 = want
+  got = np.asarray(got, np.float64)
+  assert got.shape == shape, (what, got.shape, shape)
   if got.size:
-    assert np.abs(got - want).max() <= tol * max(1.0, np.abs(want).max()), what
+    bound = tol * max(1.0, peak)
+    assert np.abs(got.ravel()[mg.sample_index(got.size)] - values).max() <= bound, what
+    assert abs(np.abs(got).max() - peak) <= bound, what
+    assert abs(np.sqrt((got * got).sum()) - l2) <= bound * np.sqrt(got.size), what
+
+
+def _w(x):
+  return None if x is None else x.astype(np.float64)
 
 
 def test_fft_convolve_shapes_paddings_delays(ref):
-  ddsp, tf = ref
-  rng = np.random.default_rng(123)
   checked = 0
-  for _ in range(24):
-    b, f = int(rng.integers(1, 3)), int(rng.choice([1, 2, 5, 10, 25]))
-    frame, s = int(rng.choice([1, 3, 16, 48, 64])), int(rng.choice([1, 2, 3, 10, 31, 64, 65, 128, 200]))
-    pad, dc = str(rng.choice(['same', 'valid'])), int(rng.choice([-1, 0, 1, 5]))
-    a = rng.standard_normal((b, f * frame)).astype(np.float32)
-    ir = rng.standard_normal((b, f, s)).astype(np.float32)
-    try:
-      want = _wide(tf, lambda: ddsp.core.fft_convolve(a, ir, padding=pad, delay_compensation=dc))
-    except Exception:  # pylint: disable=broad-except
+  for i, c in enumerate(mg.fuzz_fft_convolve_cases()):
+    want = ref['fft_convolve_%d' % i]
+    kw = dict(padding=c['padding'], delay_compensation=c['delay_compensation'])
+    if want is None:            # the reference raises on these arguments
       with pytest.raises(Exception):
-        o.fft_convolve(a.astype(np.float64), ir.astype(np.float64), padding=pad,
-                       delay_compensation=dc)
+        o.fft_convolve(_w(c['a']), _w(c['ir']), **kw)
       continue
-    got = o.fft_convolve(a.astype(np.float64), ir.astype(np.float64), padding=pad,
-                         delay_compensation=dc)
-    _close(got, want, 1e-9, ('fft_convolve', b, f, frame, s, pad, dc))
+    got = o.fft_convolve(_w(c['a']), _w(c['ir']), **kw)
+    _close(got, want, 1e-9, ('fft_convolve', c['a'].shape, c['ir'].shape, kw))
     checked += 1
   assert checked >= 12
 
 
 def test_frequency_filter_windows(ref):
-  ddsp, tf = ref
-  rng = np.random.default_rng(124)
-  for _ in range(20):
-    f, frame = int(rng.choice([1, 4, 10])), int(rng.choice([8, 32, 64]))
-    nb = int(rng.choice([2, 3, 9, 16, 33, 65, 100, 129, 130, 257]))
-    ws = int(rng.choice([0, 1, 2, 3, 7, 8, 50, 51, 64, 65, 257]))
-    a = rng.uniform(-1, 1, (1, f * frame)).astype(np.float32)
-    m = rng.uniform(0, 1, (1, f, nb)).astype(np.float32)
-    want = _wide(tf, lambda: ddsp.core.frequency_filter(a, m, window_size=ws))
-    got = o.frequency_filter(a.astype(np.float64), m.astype(np.float64), window_size=ws)
-    _close(got, want, 1e-9, ('frequency_filter', f, frame, nb, ws))
+  for i, c in enumerate(mg.fuzz_frequency_filter_cases()):
+    got = o.frequency_filter(_w(c['audio']), _w(c['magnitudes']),
+                             window_size=c['window_size'])
+    _close(got, ref['frequency_filter_%d' % i], 1e-9,
+           ('frequency_filter', c['audio'].shape, c['magnitudes'].shape, c['window_size']))
 
 
 def test_harmonic_synthesis_argument_space(ref):
-  ddsp, tf = ref
-  rng = np.random.default_rng(321)
-  for _ in range(14):
-    b, f = int(rng.integers(1, 3)), int(rng.choice([2, 5, 10, 25]))
-    hop, k = int(rng.choice([4, 16, 64, 100])), int(rng.choice([1, 3, 20, 60]))
-    method = str(rng.choice(['window', 'linear', 'nearest', 'cubic']))
-    uac, sr = bool(rng.integers(0, 2)), int(rng.choice([16000, 8000, 44100]))
-    f0 = rng.uniform(20, sr * 0.45, (b, f, 1)).astype(np.float32)
-    amp = rng.uniform(0, 1, (b, f, 1)).astype(np.float32)
-    hd = rng.uniform(0, 1, (b, f, k)).astype(np.float32) if rng.integers(0, 4) else None
-    shifts = (rng.uniform(-0.05, 0.05, (b, f, k)).astype(np.float32)
-              if hd is not None and rng.integers(0, 2) else None)
-    # tensors, so that the wide mode widens every operand (a raw float32 array in
-    # `1.0 + harmonic_shifts` would be rounded by NumPy before the shim sees it)
-    t = lambda x: None if x is None else tf.convert_to_tensor(x)  # noqa: E731
-    want = _wide(tf, lambda: ddsp.core.harmonic_synthesis(
-        t(f0), t(amp), harmonic_shifts=t(shifts), harmonic_distribution=t(hd),
-        n_samples=f * hop, sample_rate=sr, amp_resample_method=method,
-        use_angular_cumsum=uac))
-    w = lambda x: None if x is None else x.astype(np.float64)  # noqa: E731
-    got = o.harmonic_synthesis(w(f0), w(amp), harmonic_shifts=w(shifts),
-                               harmonic_distribution=w(hd), n_samples=f * hop,
-                               sample_rate=sr, amp_resample_method=method,
-                               use_angular_cumsum=uac, dtype=np.float64)
-    _close(got, want, 2e-7, ('harmonic_synthesis', b, f, hop, k, method, uac, sr))
+  for i, c in enumerate(mg.fuzz_harmonic_synthesis_cases()):
+    got = o.harmonic_synthesis(_w(c['f0']), _w(c['amp']), harmonic_shifts=_w(c['shifts']),
+                               harmonic_distribution=_w(c['hd']), n_samples=c['n_samples'],
+                               sample_rate=c['sample_rate'], amp_resample_method=c['method'],
+                               use_angular_cumsum=c['use_angular_cumsum'], dtype=np.float64)
+    _close(got, ref['harmonic_synthesis_%d' % i], 2e-7,
+           ('harmonic_synthesis', i, c['f0'].shape, c['n_samples'], c['method'],
+            c['use_angular_cumsum'], c['sample_rate']))
 
 
 def test_controls_oscillators_streaming_and_scalers(ref):
-  ddsp, tf = ref
-  rng = np.random.default_rng(999)
-  t = tf.convert_to_tensor
-  for _ in range(8):                                   # Harmonic.get_controls variants
-    f, k = int(rng.choice([3, 10])), int(rng.choice([1, 7, 40]))
-    scale, nyq, sr = bool(rng.integers(0, 2)), bool(rng.integers(0, 2)), int(rng.choice([16000, 4000]))
-    a = rng.standard_normal((1, f, 1)).astype(np.float32)
-    h = rng.standard_normal((1, f, k)).astype(np.float32)
-    f0 = rng.uniform(0, sr / 2, (1, f, 1)).astype(np.float32)
-    if not scale:
-      a, h = np.abs(a), np.abs(h)
-    syn = ddsp.synths.Harmonic(n_samples=f * 8, sample_rate=sr,
-                               scale_fn=ddsp.core.exp_sigmoid if scale else None,
-                               normalize_below_nyquist=nyq)
-    want = _wide(tf, lambda: syn.get_controls(a, h, f0))
-    got = o.harmonic_get_controls(a.astype(np.float64), h.astype(np.float64),
-                                  f0.astype(np.float64), sample_rate=sr, scale=scale,
-                                  normalize_below_nyquist=nyq, dtype=np.float64)
-    for key in ('amplitudes', 'harmonic_distribution', 'f0_hz'):
-      _close(got[key], want[key], 1e-12, ('get_controls', key, f, k, scale, nyq, sr))
-  for _ in range(8):                                   # oscillator_bank
-    b, n, k = int(rng.integers(1, 3)), int(rng.choice([50, 1000, 2500])), int(rng.choice([1, 4, 17]))
-    sr, ss, uac = int(rng.choice([16000, 8000])), bool(rng.integers(0, 2)), bool(rng.integers(0, 2))
-    fe = rng.uniform(0, sr * 0.6, (b, n, k)).astype(np.float32)
-    ae = rng.uniform(0, 1, (b, n, k)).astype(np.float32)
-    want = _wide(tf, lambda: ddsp.core.oscillator_bank(t(fe), t(ae), sample_rate=sr,
-                                                       sum_sinusoids=ss, use_angular_cumsum=uac))
-    got = o.oscillator_bank(fe.astype(np.float64), ae.astype(np.float64), sample_rate=sr,
-                            sum_sinusoids=ss, use_angular_cumsum=uac, dtype=np.float64)
-    _close(got, want, 1e-8, ('oscillator_bank', b, n, k, sr, ss, uac))
-  for _ in range(8):                                   # streaming synthesis, carried phase
-    b, f, hop = int(rng.integers(1, 3)), int(rng.choice([1, 4, 10])), int(rng.choice([16, 64]))
-    k = int(rng.choice([1, 5, 30]))
-    f0 = rng.uniform(50, 2000, (b, f, 1)).astype(np.float32)
-    amp = rng.uniform(0, 1, (b, f, 1)).astype(np.float32)
-    hd = rng.uniform(0, 1, (b, f, k)).astype(np.float32) if rng.integers(0, 3) else None
-    ph = rng.uniform(0, 6.28, (b, 1, 1)).astype(np.float32) if rng.integers(0, 2) else None
-    method = str(rng.choice(['linear', 'window']))
-    tt = lambda x: None if x is None else t(x)  # noqa: E731
-    want = _wide(tf, lambda: list(ddsp.core.streaming_harmonic_synthesis(
-        t(f0), t(amp), tt(hd), tt(ph), n_samples=f * hop, sample_rate=16000,
-        amp_resample_method=method)))
-    w = lambda x: None if x is None else x.astype(np.float64)  # noqa: E731
-    got = o.streaming_harmonic_synthesis(w(f0), w(amp), w(hd), w(ph), n_samples=f * hop,
-                                         sample_rate=16000, amp_resample_method=method,
-                                         dtype=np.float64)
-    _close(got[0], want[0], 1e-8, ('streaming audio', b, f, hop, k, method))
-    d = np.angle(np.exp(1j * (np.asarray(got[1], np.float64) - np.asarray(want[1], np.float64))))
-    assert np.abs(d).max() <= 1e-8
-  for _ in range(5):                                   # scaling functions
-    x = (4 * rng.standard_normal((2, 5, 7))).astype(np.float32)
-    ex, mv, th = float(rng.choice([10.0, 2.0, 5.0])), float(rng.choice([2.0, 1.0])), float(rng.choice([1e-7, 1e-3]))
-    _close(o.exp_sigmoid(x.astype(np.float64), ex, mv, th, dtype=np.float64),
-           _wide(tf, lambda: ddsp.core.exp_sigmoid(t(x), ex, mv, th)), 1e-12, 'exp_sigmoid')
-    depth = int(rng.choice([1, 8, 64]))
-    fr = rng.standard_normal((2, 5, 3 * depth)).astype(np.float32)
-    _close(o.frequencies_sigmoid(fr.astype(np.float64), depth=depth, dtype=np.float64),
-           _wide(tf, lambda: ddsp.core.frequencies_sigmoid(t(fr), depth=depth)), 1e-9, 'sigmoid')
-    _close(o.frequencies_softmax(fr.astype(np.float64), depth=depth, dtype=np.float64),
-           _wide(tf, lambda: ddsp.core.frequencies_softmax(t(fr), depth=depth)), 1e-9, 'softmax')
-  for _ in range(4):                                   # Sinusoidal
-    f, k, hop = int(rng.choice([5, 10])), int(rng.choice([1, 4, 9])), int(rng.choice([16, 64]))
-    a = rng.standard_normal((1, f, k)).astype(np.float32)
-    fr = rng.standard_normal((1, f, k)).astype(np.float32)
-    method = str(rng.choice(['window', 'linear']))
-    syn = ddsp.synths.Sinusoidal(n_samples=f * hop, sample_rate=16000, amp_resample_method=method)
-    want = _wide(tf, lambda: syn(t(a), t(fr)))
-    c = o.sinusoidal_get_controls(a.astype(np.float64), fr.astype(np.float64), dtype=np.float64)
-    got = o.sinusoidal_get_signal(c['amplitudes'], c['frequencies'], f * hop,
-                                  amp_resample_method=method, dtype=np.float64)
-    _close(got, want, 1e-8, ('sinusoidal', f, k, hop, method))
+  for i, (kind, c) in enumerate(mg.fuzz_misc_cases()):
+    key = '%s_%d' % (kind, i)
+    if kind == 'get_controls':
+      got = o.harmonic_get_controls(_w(c['a']), _w(c['h']), _w(c['f0']),
+                                    sample_rate=c['sample_rate'], scale=c['scale'],
+                                    normalize_below_nyquist=c['nyquist'], dtype=np.float64)
+      for name in ('amplitudes', 'harmonic_distribution', 'f0_hz'):
+        _close(got[name], ref['%s_%s' % (key, name)], 1e-12, (key, name))
+    elif kind == 'oscillator_bank':
+      got = o.oscillator_bank(_w(c['fe']), _w(c['ae']), sample_rate=c['sample_rate'],
+                              sum_sinusoids=c['sum_sinusoids'],
+                              use_angular_cumsum=c['use_angular_cumsum'], dtype=np.float64)
+      _close(got, ref[key], 1e-8, key)
+    elif kind == 'streaming':           # carried phase
+      got = o.streaming_harmonic_synthesis(_w(c['f0']), _w(c['amp']), _w(c['hd']),
+                                           _w(c['phase']), n_samples=c['n_samples'],
+                                           sample_rate=16000, amp_resample_method=c['method'],
+                                           dtype=np.float64)
+      _close(got[0], ref[key + '_audio'], 1e-8, key)
+      shape, values, _, _ = ref[key + '_phase']
+      phase = np.asarray(got[1], np.float64)
+      assert phase.shape == shape and values.size == phase.size, key
+      d = np.angle(np.exp(1j * (phase.ravel() - values)))    # on the circle
+      assert np.abs(d).max() <= 1e-8, key
+    elif kind == 'scalers':
+      _close(o.exp_sigmoid(_w(c['x']), c['exponent'], c['max_value'], c['threshold'],
+                           dtype=np.float64), ref[key + '_exp_sigmoid'], 1e-12, key)
+      _close(o.frequencies_sigmoid(_w(c['fr']), depth=c['depth'], dtype=np.float64),
+             ref[key + '_sigmoid'], 1e-9, key)
+      _close(o.frequencies_softmax(_w(c['fr']), depth=c['depth'], dtype=np.float64),
+             ref[key + '_softmax'], 1e-9, key)
+    else:                               # Sinusoidal
+      ctl = o.sinusoidal_get_controls(_w(c['a']), _w(c['fr']), dtype=np.float64)
+      got = o.sinusoidal_get_signal(ctl['amplitudes'], ctl['frequencies'], c['n_samples'],
+                                    amp_resample_method=c['method'], dtype=np.float64)
+      _close(got, ref[key], 1e-8, key)
