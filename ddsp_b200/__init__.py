@@ -14,6 +14,6 @@ from ddsp_b200 import synths
 from ddsp_b200.effects import FIRFilter, FilteredNoiseReverb, Reverb
 from ddsp_b200.host import HostDecoder
 from ddsp_b200.processors import Add, Processor, ProcessorGroup
-from ddsp_b200.synths import FilteredNoise, Harmonic, Sinusoidal
+from ddsp_b200.synths import FilteredNoise, Harmonic, Sinusoidal, Wavetable
 
 __version__ = '0.1.0'

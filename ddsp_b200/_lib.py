@@ -89,6 +89,13 @@ SIGNATURES = {
     'ddsp_b200_sinusoidal_workspace': (_sz, [_i, _i, _i]),
     'ddsp_b200_sinusoidal_forward':
         (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _f, _i, _i, _vp, _sz, _vp]),
+    'ddsp_b200_wavetable_workspace': (_sz, [_i, _i, _i, _i, _i, _i]),
+    'ddsp_b200_wavetable_forward':
+        (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _i, _i, _vp, _sz, _vp]),
+    'ddsp_b200_wavetable_backward':
+        (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _i, _vp, _sz,
+              _vp]),
+    'ddsp_b200_linear_lookup': (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _vp]),
     'ddsp_b200_add': (_i, [_vp, _vp, _vp, _i64, _vp]),
     'ddsp_b200_frame_window': (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
     'ddsp_b200_frame_window_adjoint':

@@ -260,3 +260,75 @@ def decoder_train_unfused(amps, harmonic_distribution, f0_hz, noise_magnitudes,
   mags = exp_sigmoid(noise_magnitudes + initial_bias)
   nz = FilteredNoiseFn.apply(mags, n_samples, window_size, noise, seed, offset)
   return harm + nz
+
+
+class WavetableSynthesisFn(torch.autograd.Function):
+  """core.wavetable_synthesis (core.py:1229-1282), differentiable in the
+  amplitudes and the wavetables.  scale=True: amplitudes and wavetables are RAW
+  network outputs and Wavetable.get_controls' exp_sigmoid (synths.py:212-236) is
+  part of the node, forward and backward.  Backward is
+  `ddsp_b200_wavetable_backward` (gather form, bit-reproducible).  f0 gets no
+  gradient: an f0 that requires grad is refused."""
+
+  @staticmethod
+  def forward(ctx, f0_hz, amplitudes, wavetables, n_samples, sample_rate, scale):
+    n_samples = int(n_samples)
+    b, ff, fa, _, _ = core._wavetable_shapes(f0_hz, amplitudes, wavetables, n_samples)  # pylint: disable=protected-access
+    if ff != fa:
+      raise NotImplementedError(
+          f'WavetableSynthesisFn needs f0 and amplitudes on the same frames '
+          f'(got {ff} and {fa}).')
+    f0 = core.torch_float32(f0_hz)
+    amps = core.torch_float32(amplitudes)
+    tables = core.torch_float32(wavetables)
+    tables3 = tables if tables.dim() == 3 else tables[:, None, :]
+    ctx.save_for_backward(f0, amps, tables3)
+    ctx.cfg = (n_samples, float(sample_rate), bool(scale), tuple(tables.shape))
+    out = torch.empty((b, n_samples), dtype=torch.float32, device=f0.device)
+    return core._wavetable_launch(f0, amps, tables3, n_samples, sample_rate,  # pylint: disable=protected-access
+                                  scale, out, False)
+
+  @staticmethod
+  def backward(ctx, grad_audio):
+    f0, amps, tables = ctx.saved_tensors
+    n_samples, sample_rate, scale, tshape = ctx.cfg
+    b, f = f0.shape[0], f0.shape[1]
+    r, w = tables.shape[1], tables.shape[2]
+    grad_audio = grad_audio.contiguous().to(torch.float32)
+    d_amps = torch.empty_like(amps)
+    d_tables = torch.empty_like(tables)
+    lib = _lib.load()
+    with core._on_device_of(f0, amps, tables, grad_audio):  # pylint: disable=protected-access
+      nbytes = lib.ddsp_b200_wavetable_workspace(b, f, r, w, n_samples, 1)
+      ws = torch.empty((max(nbytes, 1),), dtype=torch.uint8, device=f0.device)
+      _lib.check(lib.ddsp_b200_wavetable_backward(
+          f0.data_ptr(), amps.data_ptr(), tables.data_ptr(), grad_audio.data_ptr(),
+          d_amps.data_ptr(), d_tables.data_ptr(), b, f, r, w, n_samples, sample_rate,
+          int(scale), ws.data_ptr(), nbytes, _stream()))
+    return None, d_amps, d_tables.reshape(tshape), None, None, None
+
+
+def _refuse_f0_grad(f0_hz):
+  if isinstance(f0_hz, torch.Tensor) and f0_hz.requires_grad and torch.is_grad_enabled():
+    raise NotImplementedError(
+        'ddsp_b200 wavetable synthesis has no gradient with respect to f0_hz (the '
+        'reference models do not learn f0 through a wavetable); pass '
+        'f0_hz.detach().')
+
+
+def wavetable_synthesis(frequencies, amplitudes, wavetables, n_samples=64000,
+                        sample_rate=16000):
+  """core.wavetable_synthesis on CONTROLS with gradients to amplitudes and
+  wavetables."""
+  _refuse_f0_grad(frequencies)
+  return WavetableSynthesisFn.apply(frequencies, amplitudes, wavetables, n_samples,
+                                    sample_rate, False)
+
+
+def wavetable_train(amps_raw, wavetables_raw, f0_hz, n_samples=64000,
+                    sample_rate=16000):
+  """synths.Wavetable() (exp_sigmoid scaling) from RAW network outputs with
+  gradients to both: one forward launch, one backward pass."""
+  _refuse_f0_grad(f0_hz)
+  return WavetableSynthesisFn.apply(f0_hz, amps_raw, wavetables_raw, n_samples,
+                                    sample_rate, True)

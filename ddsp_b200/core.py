@@ -532,6 +532,161 @@ def sinusoidal_synthesis(frequencies, amplitudes, n_samples: int = 64000,
   return out
 
 
+# ----------------------------------------------------------------------------
+# Wavetable synthesis (core.py:1167-1282)
+# ----------------------------------------------------------------------------
+def linear_lookup(phase, wavetables):
+  """core.linear_lookup (core.py:1168-1209): phase [batch, n_samples] or
+  [batch, n_samples, 1]; wavetables [batch, n_wavetable] or
+  [batch, n_samples, n_wavetable] -> [batch, n_samples].
+
+  Entry n_wavetable is entry 0 and the weight on entry j is
+  relu(1 - |phase - j / n_wavetable| * n_wavetable): linear interpolation at
+  phase * n_wavetable, with entries outside [0, n_wavetable] weighing zero - so
+  a phase below 0 or above 1 fades to silence within one entry, as in the
+  reference.  One gather kernel (`ddsp_b200_linear_lookup`); inference only."""
+  sp, sw = _shape(phase), _shape(wavetables)
+  if len(sp) == 3 and sp[2] == 1:
+    sp = sp[:2]
+  if len(sp) != 2 or len(sw) not in (2, 3) or sw[0] != sp[0] or (
+      len(sw) == 3 and sw[1] not in (1, sp[1])):
+    raise ValueError(f'phase {_shape(phase)} must be [batch, n_samples(, 1)] and '
+                     f'wavetables {sw} [batch, n_wavetable] or [batch, n_samples, '
+                     'n_wavetable].')
+  b, n = sp
+  w = int(sw[-1])
+  ph = torch_float32(phase).reshape(b, n)
+  tab = torch_float32(wavetables)
+  if len(sw) == 3 and sw[1] == 1 and n != 1:
+    sw = sw[:1] + sw[2:]              # one table frame broadcasts over time
+    tab = tab.reshape(b, w)
+  _no_grad_path('linear_lookup', ph, tab)
+  out = torch.empty((b, n), dtype=torch.float32, device=ph.device)
+  with _on_device_of(ph, tab):
+    _lib.check(_lib.load().ddsp_b200_linear_lookup(
+        _ptr(ph), _ptr(tab), _ptr(out), b, n, w, int(len(sw) == 3), _stream()))
+  return out
+
+
+def harmonic_distribution_to_wavetable(harmonic_distribution, n_wavetable=2048):
+  """core.harmonic_distribution_to_wavetable (core.py:1212-1226):
+  (n_wavetable / 2) * irfft([0, hd, 0, ...]) on torch.fft (a frame-rate helper, off
+  the synthesis path).  The reference pads with n_wavetable / 2 - n_harmonics
+  zeros, which fails for more harmonics than that; this raises a ValueError."""
+  sh = _shape(harmonic_distribution)
+  if len(sh) != 3:
+    raise ValueError(f'harmonic_distribution must be [batch, time, n_harmonics], '
+                     f'got {sh}.')
+  n_pad = int(n_wavetable / 2 - sh[-1])
+  if n_pad < 0:
+    raise ValueError(f'harmonic_distribution_to_wavetable: {sh[-1]} harmonics do not '
+                     f'fit a wavetable of {n_wavetable} samples (at most '
+                     f'{int(n_wavetable) // 2}).')
+  hd = torch_float32(harmonic_distribution)
+  fft_in = torch.nn.functional.pad(hd, (1, n_pad))
+  return torch.fft.irfft(fft_in.to(torch.complex64), dim=-1) * (n_wavetable / 2)
+
+
+def _wavetable_shapes(frequencies, amplitudes, wavetables, n_samples):
+  """Shape checks and the reference's ValueErrors of wavetable_synthesis, before
+  any device work.  Returns (b, f0 frames, amp frames, table frames, W)."""
+  sf, sa, sw = _shape(frequencies), _shape(amplitudes), _shape(wavetables)
+  if len(sf) != 3 or len(sa) != 3 or sf[2] != 1 or sa[2] != 1 or sf[0] != sa[0]:
+    raise ValueError(f'frequencies {sf} and amplitudes {sa} must be '
+                     '[batch, n_frames, 1].')
+  if len(sw) not in (2, 3) or sw[0] != sf[0]:
+    raise ValueError(f'wavetables {sw} must be [batch, n_wavetable] or '
+                     '[batch, n_frames, n_wavetable].')
+  fa = sa[1]
+  if fa + 1 >= n_samples:
+    # core.py:682-685 (the amplitudes are resampled with 'window')
+    raise ValueError('Upsample with windows cannot be used for downsampling'
+                     'More input frames ({}) than output timesteps ({})'.format(
+                         fa + 1, n_samples))
+  if n_samples % fa != 0:
+    # core.py:687-693
+    raise ValueError(
+        'For upsampling, the target the number of timesteps must be divisible '
+        'by the number of input frames. (timesteps:{}, frames:{}, '
+        'add_endpoint=True).'.format(n_samples, fa + 1))
+  r = 1 if len(sw) == 2 else sw[1]
+  return sf[0], sf[1], fa, r, sw[-1]
+
+
+def _wavetable_launch(f0, amps, tables, n_samples, sample_rate, scale, out, accumulate):
+  """ddsp_b200_wavetable_forward on [B,F,1] controls (equal frame counts, F | N)
+  and [B,R,W] tables."""
+  b, f = f0.shape[0], f0.shape[1]
+  r, w = tables.shape[1], tables.shape[2]
+  lib = _lib.load()
+  with _on_device_of(f0, amps, tables, out):
+    nbytes = lib.ddsp_b200_wavetable_workspace(b, f, r, w, n_samples, 0)
+    ws = torch.empty((max(nbytes, 1),), dtype=torch.uint8, device=f0.device)
+    _lib.check(lib.ddsp_b200_wavetable_forward(
+        _ptr(f0), _ptr(amps), _ptr(tables), _ptr(out), b, f, r, w, n_samples,
+        float(sample_rate), int(bool(scale)), int(bool(accumulate)), _ptr(ws), nbytes,
+        _stream()))
+  return out
+
+
+def wavetable_synthesis(frequencies, amplitudes, wavetables, n_samples: int = 64000,
+                        sample_rate: int = 16000, out=None, accumulate: bool = False):
+  """core.wavetable_synthesis (core.py:1229-1282): frame-rate f0 [batch, frames, 1]
+  and amplitudes [batch, frames, 1], wavetables [batch, n_wavetable] (static) or
+  [batch, table_frames, n_wavetable] -> audio [batch, n_samples].
+
+  One kernel (`ddsp_b200_wavetable_forward`) reads the frame-rate tables: the
+  reference's audio-rate tables and its [batch, n_samples, n_wavetable + 1] lookup
+  weights are never formed.  The phase is the exclusive cumsum of f0 / sr mod 1,
+  accumulated exactly (64-bit fixed point).  When f0 and the amplitudes have
+  different frame counts, or n_samples is not a multiple of f0's, both are first
+  brought to audio rate with the resample kernel."""
+  n_samples = int(n_samples)
+  b, ff, fa, _, _ = _wavetable_shapes(frequencies, amplitudes, wavetables, n_samples)
+  f0 = torch_float32(frequencies)
+  amps = torch_float32(amplitudes)
+  tables = torch_float32(wavetables)
+  _no_grad_path('wavetable_synthesis', f0, amps, tables)
+  if tables.dim() == 2:
+    tables = tables[:, None, :]
+  if out is None:
+    out = torch.empty((b, n_samples), dtype=torch.float32, device=f0.device)
+    accumulate = False
+  else:
+    _check_out(out, (b, n_samples), f0)
+  if ff != fa or n_samples % ff != 0:
+    with _on_device_of(f0, amps):
+      f0 = resample(f0, n_samples)
+      amps = resample(amps, n_samples, method='window')
+  return _wavetable_launch(f0, amps, tables, n_samples, sample_rate, False, out,
+                           accumulate)
+
+
+def wavetable_raw(amplitudes, wavetables, f0_hz, n_samples: int = 64000,
+                  sample_rate: int = 16000, out=None, accumulate: bool = False):
+  """synths.Wavetable()(...) with the default exp_sigmoid scaling from RAW network
+  outputs in one launch: exp_sigmoid is applied to the amplitudes and to each
+  table row as it lands in shared memory (bit-identical to get_signal of
+  get_controls).  Needs f0 and amplitudes on the same frames, a multiple of which
+  n_samples is, and 3-D tables."""
+  n_samples = int(n_samples)
+  b, ff, fa, _, _ = _wavetable_shapes(f0_hz, amplitudes, wavetables, n_samples)
+  if ff != fa or len(_shape(wavetables)) != 3:
+    raise ValueError('wavetable_raw needs f0 and amplitudes on the same frames and '
+                     '[batch, frames, n_wavetable] tables.')
+  f0 = torch_float32(f0_hz)
+  amps = torch_float32(amplitudes)
+  tables = torch_float32(wavetables)
+  _no_grad_path('wavetable_raw', f0, amps, tables)
+  if out is None:
+    out = torch.empty((b, n_samples), dtype=torch.float32, device=f0.device)
+    accumulate = False
+  else:
+    _check_out(out, (b, n_samples), f0)
+  return _wavetable_launch(f0, amps, tables, n_samples, sample_rate, True, out,
+                           accumulate)
+
+
 def harmonic_synthesis(frequencies,
                        amplitudes,
                        harmonic_shifts=None,

@@ -20,6 +20,7 @@
 #include "controls_bwd.cuh"
 #include "oscbank.cuh"
 #include "sinusoidal.cuh"
+#include "wavetable.cuh"
 #include "longconv.cuh"
 #include "spectral.cuh"
 
@@ -1039,6 +1040,171 @@ int ddsp_b200_sinusoidal_forward(const float* frequencies, const float* amplitud
         sample_rate * 0.5f, accumulate);
   }
   DDSP_CHECK_LAUNCH("sinusoidal_forward(apply)");
+  return 0;
+}
+
+// ---- wavetable synthesis (wavetable.cuh) -------------------------------------
+static inline size_t wt_align(size_t x) { return (x + 255) & ~(size_t)255; }
+
+// Backward warp tasks walk at most kWtSeg samples; a row is read by the samples
+// of two table intervals (at most 2 ceil(N / R)).
+static int wt_nseg(int R, int N) {
+  const long long span = 2 * (((long long)N + R - 1) / R);
+  return (int)std::max<long long>(1, (span + kWtSeg - 1) / kWtSeg);
+}
+
+// Backward CTA: nw warp tasks, nw + 1 staged rows and nw accumulator rows.
+static int wt_bwd_warps(int W) {
+  for (int nw = 4; nw >= 1; nw >>= 1)
+    if ((size_t)(2 * nw + 1) * W * sizeof(float) <= kMaxDynSmem) return nw;
+  return 0;
+}
+
+size_t ddsp_b200_wavetable_workspace(int B, int F, int R, int W, int N, int backward) {
+  if (B <= 0 || F <= 0 || R <= 0 || W <= 0 || N <= 0) return 0;
+  size_t n = 256 + wt_align(sizeof(WtRec) * (size_t)B * F);
+  if (backward) {
+    n += wt_align(sizeof(float) * (size_t)B * N);
+    const int nseg = wt_nseg(R, N);
+    if (nseg > 1) n += wt_align(sizeof(float) * (size_t)B * R * nseg * W);
+  }
+  return n;
+}
+
+static int wt_check(const char* name, int B, int F, int R, int W, int N,
+                    float sample_rate) {
+  DDSP_REQUIRE(B >= 0 && F >= 1 && R >= 1 && W >= 1 && N >= 1, DDSP_B200_E_INVALID,
+               "%s: bad shape B=%d F=%d R=%d W=%d N=%d", name, B, F, R, W, N);
+  DDSP_REQUIRE(N % F == 0, DDSP_B200_E_INVALID,
+               "%s: n_samples (%d) must be divisible by the number of frames (%d)",
+               name, N, F);
+  DDSP_REQUIRE(sample_rate > 0.f, DDSP_B200_E_INVALID,
+               "%s: sample_rate must be positive", name);
+  DDSP_REQUIRE(B <= 65535, DDSP_B200_E_INVALID,
+               "%s: B=%d exceeds the 65535 grid limit", name, B);
+  return 0;
+}
+
+int ddsp_b200_wavetable_forward(const float* f0_hz, const float* amps,
+                                const float* tables, float* audio, int B, int F, int R,
+                                int W, int N, float sample_rate, int scale,
+                                int accumulate, void* workspace, size_t workspace_bytes,
+                                void* stream) {
+  DDSP_REQUIRE(f0_hz && amps && tables && audio, DDSP_B200_E_INVALID,
+               "wavetable_forward: null pointer");
+  int rc = wt_check("wavetable_forward", B, F, R, W, N, sample_rate);
+  if (rc) return rc;
+  if (B == 0) return 0;
+  const int ring = (int)std::min<size_t>(4, kMaxDynSmem / (sizeof(float) * (size_t)W));
+  DDSP_REQUIRE(ring >= 2, DDSP_B200_E_UNSUPPORTED,
+               "wavetable_forward: a wavetable of %d samples does not fit two rows of "
+               "shared memory", W);
+  const size_t need = ddsp_b200_wavetable_workspace(B, F, R, W, N, 0);
+  DDSP_REQUIRE(workspace != nullptr && workspace_bytes >= need, DDSP_B200_E_WORKSPACE,
+               "wavetable_forward: workspace of %zu B needed, %zu given", need,
+               workspace_bytes);
+  WtRec* recs = reinterpret_cast<WtRec*>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
+  cudaStream_t st = (cudaStream_t)stream;
+  const int hop = N / F;
+  wt_phase_records<<<B, 32, 0, st>>>(f0_hz, recs, F, hop, 1.0 / (double)sample_rate);
+  DDSP_CHECK_LAUNCH("wavetable_forward(phase records)");
+
+  WtParams p;
+  p.tables = tables; p.amps = amps; p.rec = recs; p.out = audio;
+  p.B = B; p.F = F; p.R = R; p.W = W; p.N = N; p.hop = hop;
+  p.ring = ring; p.scale = scale ? 1 : 0; p.accumulate = accumulate ? 1 : 0;
+  p.inv_hop = 1.0f / (float)hop;
+  p.inv_n = 1.0f / (float)N;
+  // ~16 table intervals per CTA, enough CTAs to cover the chip
+  const long long spi = ((long long)N + R - 1) / R;
+  long long tc = std::min<long long>(8192, std::max<long long>(512, 16 * spi));
+  while (tc > 512 && (long long)B * ((N + tc - 1) / tc) < 4ll * kNumSMs) tc /= 2;
+  p.t_chunk = (int)tc;
+  const size_t smem = 128 + sizeof(float) * (size_t)ring * W;
+  dim3 grid((unsigned)((N + tc - 1) / tc), B);
+  const bool tma = (W % 4 == 0) && (((uintptr_t)tables & 15) == 0);
+  if (tma) {
+    rc = set_smem(wt_forward<true>, smem, "wavetable_forward");
+    if (rc) return rc;
+    wt_forward<true><<<grid, kWtThreads, smem, st>>>(p);
+  } else {
+    rc = set_smem(wt_forward<false>, smem, "wavetable_forward");
+    if (rc) return rc;
+    wt_forward<false><<<grid, kWtThreads, smem, st>>>(p);
+  }
+  DDSP_CHECK_LAUNCH("wavetable_forward");
+  return 0;
+}
+
+int ddsp_b200_wavetable_backward(const float* f0_hz, const float* amps,
+                                 const float* tables, const float* grad_audio,
+                                 float* d_amps, float* d_tables, int B, int F, int R,
+                                 int W, int N, float sample_rate, int scale,
+                                 void* workspace, size_t workspace_bytes, void* stream) {
+  DDSP_REQUIRE(f0_hz && amps && tables && grad_audio && d_amps && d_tables,
+               DDSP_B200_E_INVALID, "wavetable_backward: null pointer");
+  int rc = wt_check("wavetable_backward", B, F, R, W, N, sample_rate);
+  if (rc) return rc;
+  if (B == 0) return 0;
+  const int nw = wt_bwd_warps(W);
+  DDSP_REQUIRE(nw > 0, DDSP_B200_E_UNSUPPORTED,
+               "wavetable_backward: a wavetable of %d samples needs more shared memory "
+               "than one CTA has", W);
+  const size_t need = ddsp_b200_wavetable_workspace(B, F, R, W, N, 1);
+  DDSP_REQUIRE(workspace != nullptr && workspace_bytes >= need, DDSP_B200_E_WORKSPACE,
+               "wavetable_backward: workspace of %zu B needed, %zu given", need,
+               workspace_bytes);
+  uintptr_t base = ((uintptr_t)workspace + 255) & ~(uintptr_t)255;
+  WtRec* recs = reinterpret_cast<WtRec*>(base);
+  base += wt_align(sizeof(WtRec) * (size_t)B * F);
+  float* gl = reinterpret_cast<float*>(base);
+  base += wt_align(sizeof(float) * (size_t)B * N);
+  const int nseg = wt_nseg(R, N);
+  float* parts = nseg > 1 ? reinterpret_cast<float*>(base) : nullptr;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int hop = N / F;
+  wt_phase_records<<<B, 32, 0, st>>>(f0_hz, recs, F, hop, 1.0 / (double)sample_rate);
+  DDSP_CHECK_LAUNCH("wavetable_backward(phase records)");
+
+  WtBwdParams p;
+  p.tables = tables; p.amps = amps; p.rec = recs; p.grad = grad_audio; p.gl = gl;
+  p.d_tables = d_tables; p.parts = parts;
+  p.B = B; p.F = F; p.R = R; p.W = W; p.N = N; p.hop = hop;
+  p.nseg = nseg; p.nw = nw; p.scale = scale ? 1 : 0;
+  p.inv_hop = 1.0f / (float)hop;
+  p.inv_n = 1.0f / (float)N;
+  const long long n_tasks = (long long)R * nseg;
+  DDSP_REQUIRE((n_tasks + nw - 1) / nw < (1ll << 31), DDSP_B200_E_INVALID,
+               "wavetable_backward: too many table rows");
+  const size_t smem = sizeof(float) * (size_t)(2 * nw + 1) * W;
+  rc = set_smem(wt_backward, smem, "wavetable_backward");
+  if (rc) return rc;
+  wt_backward<<<dim3((unsigned)((n_tasks + nw - 1) / nw), B), 32 * nw, smem, st>>>(p);
+  DDSP_CHECK_LAUNCH("wavetable_backward");
+  if (nseg > 1) {
+    const long long n = (long long)B * R * W;
+    wt_reduce_parts<<<grid_for(n, 256), 256, 0, st>>>(parts, tables, d_tables,
+                                                      (long long)B * R, nseg, W,
+                                                      p.scale);
+    DDSP_CHECK_LAUNCH("wavetable_backward(partial rows)");
+  }
+  const long long warps = (long long)B * F;
+  wt_amp_grad<<<(unsigned)((warps * 32 + 255) / 256), 256, 0, st>>>(
+      gl, amps, d_amps, B, F, N, hop, p.inv_hop, p.scale);
+  DDSP_CHECK_LAUNCH("wavetable_backward(amplitudes)");
+  return 0;
+}
+
+int ddsp_b200_linear_lookup(const float* phase, const float* tables, float* out, int B,
+                            int N, int W, int per_sample, void* stream) {
+  DDSP_REQUIRE(phase && tables && out, DDSP_B200_E_INVALID, "linear_lookup: null pointer");
+  DDSP_REQUIRE(B >= 0 && N >= 0 && W >= 1, DDSP_B200_E_INVALID,
+               "linear_lookup: bad shape B=%d N=%d W=%d", B, N, W);
+  const long long total = (long long)B * N;
+  if (total == 0) return 0;
+  wt_linear_lookup<<<grid_for(total, 256), 256, 0, (cudaStream_t)stream>>>(
+      phase, tables, out, B, N, W, per_sample ? 1 : 0);
+  DDSP_CHECK_LAUNCH("linear_lookup");
   return 0;
 }
 

@@ -110,6 +110,59 @@ class FilteredNoise(processors.Processor):
         out=out, accumulate=accumulate)
 
 
+class Wavetable(processors.Processor):
+  """Synthesize audio from a series of wavetables (synths.py:199-257).
+
+  get_signal passes the frame-rate tables straight to one fused kernel
+  (`ddsp_b200_wavetable_forward`); the reference's audio-rate tables
+  [batch, n_samples, n_wavetable] never exist.  Called for the signal only with
+  the default exp_sigmoid scaling, the processor runs get_controls inside that
+  kernel (one launch from raw network outputs)."""
+
+  def __init__(self,
+               n_samples=64000,
+               sample_rate=16000,
+               scale_fn=core.exp_sigmoid,
+               name='wavetable'):
+    super().__init__(name=name)
+    self.n_samples = n_samples
+    self.sample_rate = sample_rate
+    self.scale_fn = scale_fn
+
+  def call(self, amplitudes, wavetables, f0_hz, return_outputs_dict=False, **kwargs):
+    for k in ['training', 'mask']:
+      kwargs.pop(k, None)
+    sa, sw, sf = core._shape(amplitudes), core._shape(wavetables), core._shape(f0_hz)  # pylint: disable=protected-access
+    if (not return_outputs_dict and not kwargs and self.scale_fn is core.exp_sigmoid
+        and len(sw) == 3 and len(sa) == 3 and len(sf) == 3 and sa[:2] == sf[:2]):
+      return core.wavetable_raw(amplitudes, wavetables, f0_hz,
+                                n_samples=self.n_samples, sample_rate=self.sample_rate)
+    return super().call(amplitudes, wavetables, f0_hz,
+                        return_outputs_dict=return_outputs_dict, **kwargs)
+
+  def get_controls(self, amplitudes, wavetables, f0_hz):
+    """synths.py:212-236: scale_fn on the amplitudes and the wavetables."""
+    if self.scale_fn is not None:
+      amplitudes = self.scale_fn(core.torch_float32(amplitudes))
+      wavetables = self.scale_fn(core.torch_float32(wavetables))
+    return {'amplitudes': amplitudes,
+            'wavetables': wavetables,
+            'f0_hz': f0_hz}
+
+  def get_signal(self, amplitudes, wavetables, f0_hz, out=None, accumulate=False):
+    """synths.py:238-257.  The reference resamples 3-D tables to n_samples before
+    wavetable_synthesis (which then resamples n_samples to n_samples, the
+    identity): the kernel interpolates the frame-rate tables itself.  A 2-D table
+    [batch, n_wavetable] is resampled along its only axis into a static table of
+    n_samples entries, as in the reference."""
+    if len(core._shape(wavetables)) == 2:  # pylint: disable=protected-access
+      wavetables = core.resample(wavetables, self.n_samples)
+    return core.wavetable_synthesis(f0_hz, amplitudes, wavetables,
+                                    n_samples=self.n_samples,
+                                    sample_rate=self.sample_rate, out=out,
+                                    accumulate=accumulate)
+
+
 class Sinusoidal(processors.Processor):
   """Bank of arbitrary sinusoidal oscillators (synths.py:260-323).
 

@@ -305,6 +305,36 @@ int ddsp_b200_sinusoidal_forward(const float* frequencies, const float* amplitud
                                  void* workspace, size_t workspace_bytes,
                                  void* stream);
 
+/* Wavetable synthesis: core.wavetable_synthesis / synths.Wavetable.get_signal
+ * (core.py:1212-1282, synths.py:238-257) in one pass over the frame-rate tables.
+ * f0_hz, amps [B,F] (hop N/F, N % F == 0; F == N: audio-rate controls, hop 1),
+ * tables [B,R,W]: R table frames linearly interpolated in time (src = t R / N,
+ * last frame held); R == 1 is a static table.  The phase is the EXCLUSIVE cumsum
+ * of f0/sr mod 1 (64-bit fixed point), amps are Hann-upsampled ('window').
+ * scale != 0: amps and tables are raw network outputs and exp_sigmoid
+ * (Wavetable.get_controls, synths.py:212-236) is applied inside the kernel, with
+ * the same device function as ddsp_b200_noise_controls.
+ * workspace: ddsp_b200_wavetable_workspace(B,F,R,W,N,0) bytes (forward) or
+ * (...,1) (backward).
+ * backward: grad_audio [B,N] -> d_amps [B,F], d_tables [B,R,W] (w.r.t. the raw
+ * inputs when scale != 0); deterministic, every element written once.  f0 gets
+ * no gradient. */
+size_t ddsp_b200_wavetable_workspace(int B, int F, int R, int W, int N, int backward);
+int ddsp_b200_wavetable_forward(const float* f0_hz, const float* amps,
+                                const float* tables, float* audio, int B, int F, int R,
+                                int W, int N, float sample_rate, int scale,
+                                int accumulate, void* workspace, size_t workspace_bytes,
+                                void* stream);
+int ddsp_b200_wavetable_backward(const float* f0_hz, const float* amps,
+                                 const float* tables, const float* grad_audio,
+                                 float* d_amps, float* d_tables, int B, int F, int R,
+                                 int W, int N, float sample_rate, int scale,
+                                 void* workspace, size_t workspace_bytes, void* stream);
+/* core.linear_lookup (core.py:1168-1209): phase [B,N] (any value), tables [B,W]
+ * (per_sample = 0) or [B,N,W] (per_sample = 1) -> out [B,N]. */
+int ddsp_b200_linear_lookup(const float* phase, const float* tables, float* out, int B,
+                            int N, int W, int per_sample, void* stream);
+
 /* core.resample / core.upsample_with_windows (core.py:573-714) stand-alone:
  * in [B,F,C] -> out [B,N,C].  method: 0 'window', 1 'linear', 2 'nearest',
  * 3 'cubic' (tf.compat.v1 bicubic, Keys A = -0.75).  add_endpoint as in the
