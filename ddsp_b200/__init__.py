@@ -11,7 +11,7 @@ from ddsp_b200 import effects
 from ddsp_b200 import host
 from ddsp_b200 import processors
 from ddsp_b200 import synths
-from ddsp_b200.effects import FIRFilter, FilteredNoiseReverb, Reverb
+from ddsp_b200.effects import FIRFilter, FilteredNoiseReverb, ModDelay, Reverb
 from ddsp_b200.host import HostDecoder
 from ddsp_b200.processors import Add, Processor, ProcessorGroup
 from ddsp_b200.synths import FilteredNoise, Harmonic, Sinusoidal, Wavetable

@@ -34,6 +34,7 @@ _u64 = ctypes.c_uint64
 _f = ctypes.c_float
 _vp = ctypes.c_void_p
 _sz = ctypes.c_size_t
+_d = ctypes.c_double
 
 # name -> (restype, argtypes); mirrors include/ddsp_b200.h one to one.
 SIGNATURES = {
@@ -96,6 +97,13 @@ SIGNATURES = {
         (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _f, _i, _vp, _sz,
               _vp]),
     'ddsp_b200_linear_lookup': (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _vp]),
+    'ddsp_b200_mod_delay_workspace': (_sz, [_i, _i, _i]),
+    'ddsp_b200_mod_delay_forward':
+        (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _d, _d, _i, _i, _vp]),
+    'ddsp_b200_mod_delay_backward':
+        (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _d, _d, _i, _i, _vp, _sz,
+              _vp]),
+    'ddsp_b200_sigmoid': (_i, [_vp, _vp, _i64, _vp]),
     'ddsp_b200_add': (_i, [_vp, _vp, _vp, _i64, _vp]),
     'ddsp_b200_frame_window': (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
     'ddsp_b200_frame_window_adjoint':

@@ -332,3 +332,73 @@ def wavetable_train(amps_raw, wavetables_raw, f0_hz, n_samples=64000,
   _refuse_f0_grad(f0_hz)
   return WavetableSynthesisFn.apply(f0_hz, amps_raw, wavetables_raw, n_samples,
                                     sample_rate, True)
+
+
+class ModDelayFn(torch.autograd.Function):
+  """core.variable_length_delay (core.py:1285-1313) and effects.ModDelay's
+  signal (effects.py:367-393), differentiable in the audio, the gain and the
+  phase.  gain may be None (the bare delay).  scale=True: gain and phase are RAW
+  network outputs and ModDelay.get_controls' exp_sigmoid / sigmoid are part of
+  the node, forward and backward.  Backward is `ddsp_b200_mod_delay_backward`:
+  d audio is the transpose of the two-tap gather, summed in 64-bit fixed point
+  (bit-reproducible); d phase is g gain L (e_{j+1} - e_j) times the phase map's
+  slope, and it jumps where the position crosses an integer."""
+
+  @staticmethod
+  def forward(ctx, audio, gain, phase, max_length, phase_scale, phase_offset, scale,
+              add_dry):
+    name = 'ModDelay' if gain is not None else 'variable_length_delay'
+    max_length = core._check_max_length(name, max_length)  # pylint: disable=protected-access
+    controls = {'phase': phase} if gain is None else {'gain': gain, 'phase': phase}
+    b, n = core._delay_controls(name, audio, controls)  # pylint: disable=protected-access
+    x = core.torch_float32(audio)
+    g = None if gain is None else core.torch_float32(gain).reshape(b, n)
+    ph = core.torch_float32(phase).reshape(b, n)
+    ctx.save_for_backward(x, g, ph)
+    ctx.cfg = (max_length, float(phase_scale), float(phase_offset), bool(scale),
+               bool(add_dry), None if gain is None else tuple(gain.shape),
+               tuple(phase.shape))
+    return core._mod_delay_launch(x, g, ph, max_length, phase_scale, phase_offset,  # pylint: disable=protected-access
+                                  scale, add_dry)
+
+  @staticmethod
+  def backward(ctx, grad_out):
+    x, g, ph = ctx.saved_tensors
+    max_length, phase_scale, phase_offset, scale, add_dry, gshape, pshape = ctx.cfg
+    b, n = x.shape
+    grad_out = grad_out.contiguous().to(torch.float32)
+    d_audio = torch.empty_like(x)
+    d_gain = None if g is None else torch.empty_like(g)
+    d_phase = torch.empty_like(ph)
+    lib = _lib.load()
+    with core._on_device_of(x, g, ph, grad_out):  # pylint: disable=protected-access
+      nbytes = lib.ddsp_b200_mod_delay_workspace(b, n, max_length)
+      ws = torch.empty((max(nbytes, 1),), dtype=torch.uint8, device=x.device)
+      _lib.check(lib.ddsp_b200_mod_delay_backward(
+          x.data_ptr(), 0 if g is None else g.data_ptr(), ph.data_ptr(),
+          grad_out.data_ptr(), d_audio.data_ptr(),
+          0 if d_gain is None else d_gain.data_ptr(), d_phase.data_ptr(), b, n,
+          max_length, phase_scale, phase_offset, int(scale), int(add_dry),
+          ws.data_ptr(), nbytes, _stream()))
+    if d_gain is not None:
+      d_gain = d_gain.reshape(gshape)
+    return (d_audio, d_gain, d_phase.reshape(pshape), None, None, None, None, None)
+
+
+def variable_length_delay(phase, audio, max_length=512):
+  """core.variable_length_delay on controls with gradients to the phase and the
+  audio."""
+  return ModDelayFn.apply(audio, None, phase, max_length, 1.0, 0.0, False, False)
+
+
+def mod_delay_train(audio, gain_raw, phase_raw, center_ms=15.0, depth_ms=10.0,
+                    sample_rate=16000, add_dry=True):
+  """effects.ModDelay() (exp_sigmoid gain, sigmoid phase) from RAW network outputs
+  with gradients to the audio and both controls: one forward launch, one backward
+  pass.  The audio's gradient reaches the synthesizer upstream."""
+  from ddsp_b200 import effects  # local import: effects imports core only
+  md = effects.ModDelay(center_ms=center_ms, depth_ms=depth_ms, sample_rate=sample_rate,
+                        add_dry=add_dry)
+  max_length, depth_phase, center_phase = md.delay_map()
+  return ModDelayFn.apply(audio, gain_raw, phase_raw, max_length, depth_phase,
+                          center_phase, True, add_dry)

@@ -165,6 +165,21 @@ def exp_sigmoid(x, exponent=10.0, max_value=2.0, threshold=1e-7):
   return max_value * torch.sigmoid(x)**float(np.log(exponent)) + threshold
 
 
+def sigmoid(x):
+  """tf.nn.sigmoid, the default phase_scale_fn of effects.ModDelay
+  (effects.py:331-344): 1 / (1 + e^-x) in the CUDA kernel `ddsp_b200_sigmoid`.
+  Its device function is the one ModDelay's one-launch path applies to raw
+  outputs, so both routes give the same bits.  An input that requires grad goes
+  through torch.sigmoid."""
+  x = torch_float32(x)
+  if torch.is_grad_enabled() and x.requires_grad:
+    return torch.sigmoid(x)
+  out = torch.empty_like(x)
+  with _on_device_of(x):
+    _lib.check(_lib.load().ddsp_b200_sigmoid(_ptr(x), _ptr(out), x.numel(), _stream()))
+  return out
+
+
 # ----------------------------------------------------------------------------
 # Frequency scaling of network outputs (core.py:207-348, 414-508) - frame-rate
 # torch ops (a few thousand elements per item), device-agnostic.
@@ -685,6 +700,79 @@ def wavetable_raw(amplitudes, wavetables, f0_hz, n_samples: int = 64000,
     _check_out(out, (b, n_samples), f0)
   return _wavetable_launch(f0, amps, tables, n_samples, sample_rate, True, out,
                            accumulate)
+
+
+# ----------------------------------------------------------------------------
+# Variable-length delay (core.py:1285-1313) and ModDelay's signal
+# ----------------------------------------------------------------------------
+def _delay_controls(name, audio, controls):
+  """Shape checks of the delay before any device work: audio [batch, n_samples],
+  each control [batch, n_samples] or [batch, n_samples, 1].  Returns (b, n)."""
+  sa = _shape(audio)
+  if len(sa) != 2:
+    raise ValueError(f'{name}: audio must be [batch, n_samples], got {sa}.')
+  for key, x in controls.items():
+    sx = _shape(x)
+    if len(sx) == 3 and sx[2] == 1:
+      sx = sx[:2]
+    if sx != sa:
+      raise ValueError(f'{name}: {key} {_shape(x)} must be [batch, n_samples] or '
+                       f'[batch, n_samples, 1] with audio {sa}.')
+  return sa
+
+
+def _check_max_length(name, max_length):
+  if int(max_length) != max_length or int(max_length) < 1:
+    raise ValueError(f'{name}: max_length must be an integer >= 1, got {max_length}.')
+  return int(max_length)
+
+
+def _mod_delay_launch(audio, gain, phase, max_length, phase_scale, phase_offset,
+                      scale, add_dry):
+  """ddsp_b200_mod_delay_forward on checked inputs; gain may be None."""
+  b, n = audio.shape
+  out = torch.empty((b, n), dtype=torch.float32, device=audio.device)
+  with _on_device_of(audio, gain, phase):
+    _lib.check(_lib.load().ddsp_b200_mod_delay_forward(
+        _ptr(audio), _ptr(gain), _ptr(phase), _ptr(out), b, n, int(max_length),
+        float(phase_scale), float(phase_offset), int(bool(scale)), int(bool(add_dry)),
+        _stream()))
+  return out
+
+
+def variable_length_delay(phase, audio, max_length: int = 512):
+  """core.variable_length_delay (core.py:1285-1313): phase [batch, n_samples(, 1)],
+  audio [batch, n_samples] -> [batch, n_samples].
+
+  Sample n reads its own history e_k = audio[n - k] (0 <= k < max_length, zero
+  before the start) with linear_lookup's rule at phase * max_length; entry
+  max_length is entry 0, so phase 1 gives the undelayed sample and a phase further
+  outside [0, 1] is silent, as in the reference.  One kernel
+  (`ddsp_b200_mod_delay_forward`); the reference's [batch, n_samples, max_length]
+  frames are never formed.  Inference only (see autograd.variable_length_delay)."""
+  max_length = _check_max_length('variable_length_delay', max_length)
+  b, n = _delay_controls('variable_length_delay', audio, {'phase': phase})
+  ph = torch_float32(phase).reshape(b, n)
+  x = torch_float32(audio)
+  _no_grad_path('variable_length_delay', ph, x)
+  return _mod_delay_launch(x, None, ph, max_length, 1.0, 0.0, False, False)
+
+
+def mod_delay(audio, gain, phase, max_length, phase_scale, phase_offset,
+              add_dry=True, scale=False):
+  """effects.ModDelay.get_signal (effects.py:369-393) in one launch:
+  variable_length_delay(phase * phase_scale + phase_offset, audio, max_length)
+  * gain (+ audio with add_dry).  scale=True: gain and phase are raw network
+  outputs, and exp_sigmoid / sigmoid (ModDelay.get_controls' defaults) run inside
+  the kernel, bit-identical to applying core.exp_sigmoid / core.sigmoid first."""
+  max_length = _check_max_length('ModDelay', max_length)
+  b, n = _delay_controls('ModDelay', audio, {'gain': gain, 'phase': phase})
+  x = torch_float32(audio)
+  g = torch_float32(gain).reshape(b, n)
+  ph = torch_float32(phase).reshape(b, n)
+  _no_grad_path('mod_delay', x, g, ph)
+  return _mod_delay_launch(x, g, ph, max_length, phase_scale, phase_offset, scale,
+                           add_dry)
 
 
 def harmonic_synthesis(frequencies,

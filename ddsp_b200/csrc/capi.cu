@@ -21,6 +21,7 @@
 #include "oscbank.cuh"
 #include "sinusoidal.cuh"
 #include "wavetable.cuh"
+#include "mod_delay.cuh"
 #include "longconv.cuh"
 #include "spectral.cuh"
 
@@ -1205,6 +1206,119 @@ int ddsp_b200_linear_lookup(const float* phase, const float* tables, float* out,
   wt_linear_lookup<<<grid_for(total, 256), 256, 0, (cudaStream_t)stream>>>(
       phase, tables, out, B, N, W, per_sample ? 1 : 0);
   DDSP_CHECK_LAUNCH("linear_lookup");
+  return 0;
+}
+
+// ---- modulated delay (mod_delay.cuh) -----------------------------------------
+static int md_tiles(int N) { return (N + kMdTile - 1) / kMdTile; }
+
+size_t ddsp_b200_mod_delay_workspace(int B, int N, int L) {
+  if (B <= 0 || N <= 0 || L <= 0) return 0;
+  const size_t tiles = (size_t)md_tiles(N);
+  const size_t H = (size_t)std::min(L, kMdTile);
+  return 256 + wt_align(sizeof(float) * (size_t)B * tiles) + wt_align(sizeof(int) * (size_t)B) +
+         sizeof(unsigned long long) * (size_t)B * tiles * H;
+}
+
+static int md_setup(const char* name, MdParams& p, const float* audio, const float* gain,
+                    const float* phase, int B, int N, int L, double phase_scale,
+                    double phase_offset, int scale, int add_dry) {
+  DDSP_REQUIRE(audio && phase, DDSP_B200_E_INVALID, "%s: null pointer", name);
+  DDSP_REQUIRE(B >= 0 && N >= 1 && L >= 1, DDSP_B200_E_INVALID,
+               "%s: bad shape B=%d N=%d max_length=%d", name, B, N, L);
+  DDSP_REQUIRE(B <= 65535, DDSP_B200_E_INVALID, "%s: B=%d exceeds the 65535 grid limit",
+               name, B);
+  DDSP_REQUIRE(N <= INT32_MAX - kMdTile, DDSP_B200_E_INVALID, "%s: N=%d too long", name, N);
+  p = MdParams{};
+  p.audio = audio; p.gain = gain; p.phase = phase;
+  p.B = B; p.N = N; p.L = L;
+  p.H = std::min(L, kMdTile);
+  p.tiles = md_tiles(N);
+  p.p_scale = phase_scale * (double)L;
+  p.p_offset = phase_offset * (double)L;
+  p.scale = scale ? 1 : 0;
+  p.add_dry = add_dry ? 1 : 0;
+  return 0;
+}
+
+int ddsp_b200_mod_delay_forward(const float* audio, const float* gain, const float* phase,
+                                float* out, int B, int N, int L, double phase_scale,
+                                double phase_offset, int scale, int add_dry,
+                                void* stream) {
+  MdParams p;
+  int rc = md_setup("mod_delay_forward", p, audio, gain, phase, B, N, L, phase_scale,
+                    phase_offset, scale, add_dry);
+  if (rc) return rc;
+  DDSP_REQUIRE(out, DDSP_B200_E_INVALID, "mod_delay_forward: null pointer");
+  if (B == 0) return 0;
+  p.out = out;
+  cudaStream_t st = (cudaStream_t)stream;
+  const dim3 grid((unsigned)p.tiles, (unsigned)B);
+  if (L <= kMdStageMax) {
+    const size_t smem = sizeof(float) * ((size_t)kMdTile + L - 1);
+    rc = set_smem(md_forward<true>, smem, "mod_delay_forward");
+    if (rc) return rc;
+    md_forward<true><<<grid, kMdThreads, smem, st>>>(p);
+  } else {
+    md_forward<false><<<grid, kMdThreads, 0, st>>>(p);
+  }
+  DDSP_CHECK_LAUNCH("mod_delay_forward");
+  return 0;
+}
+
+int ddsp_b200_mod_delay_backward(const float* audio, const float* gain, const float* phase,
+                                 const float* grad_out, float* d_audio, float* d_gain,
+                                 float* d_phase, int B, int N, int L, double phase_scale,
+                                 double phase_offset, int scale, int add_dry,
+                                 void* workspace, size_t workspace_bytes, void* stream) {
+  MdParams p;
+  int rc = md_setup("mod_delay_backward", p, audio, gain, phase, B, N, L, phase_scale,
+                    phase_offset, scale, add_dry);
+  if (rc) return rc;
+  DDSP_REQUIRE(grad_out && d_audio && d_phase && (d_gain || !gain), DDSP_B200_E_INVALID,
+               "mod_delay_backward: null pointer");
+  if (B == 0) return 0;
+  const size_t need = ddsp_b200_mod_delay_workspace(B, N, L);
+  DDSP_REQUIRE(workspace != nullptr && workspace_bytes >= need, DDSP_B200_E_WORKSPACE,
+               "mod_delay_backward: workspace of %zu B needed, %zu given", need,
+               workspace_bytes);
+  uintptr_t base = ((uintptr_t)workspace + 255) & ~(uintptr_t)255;
+  p.tmax = reinterpret_cast<float*>(base);
+  base += wt_align(sizeof(float) * (size_t)B * p.tiles);
+  p.kexp = reinterpret_cast<int*>(base);
+  base += wt_align(sizeof(int) * (size_t)B);
+  p.halo = reinterpret_cast<unsigned long long*>(base);
+  p.grad = grad_out; p.out = d_audio; p.d_gain = gain ? d_gain : nullptr; p.d_phase = d_phase;
+  cudaStream_t st = (cudaStream_t)stream;
+  const dim3 grid((unsigned)p.tiles, (unsigned)B);
+  md_bwd_max<<<grid, kMdThreads, 0, st>>>(p);
+  DDSP_CHECK_LAUNCH("mod_delay_backward(max)");
+  size_t smem = sizeof(unsigned long long) * kMdTile;
+  if (L <= kMdStageMax) {
+    smem += sizeof(float) * ((size_t)kMdTile + L - 1);
+    rc = set_smem(md_backward<true>, smem, "mod_delay_backward");
+    if (rc) return rc;
+    md_backward<true><<<grid, kMdThreads, smem, st>>>(p);
+  } else {
+    rc = set_smem(md_backward<false>, smem, "mod_delay_backward");
+    if (rc) return rc;
+    md_backward<false><<<grid, kMdThreads, smem, st>>>(p);
+  }
+  DDSP_CHECK_LAUNCH("mod_delay_backward");
+  if (p.tiles > 1) {
+    const long long n = (long long)B * (p.tiles - 1) * p.H;
+    md_bwd_finish<<<grid_for(n, 256), 256, 0, st>>>(p);
+    DDSP_CHECK_LAUNCH("mod_delay_backward(halo)");
+  }
+  return 0;
+}
+
+int ddsp_b200_sigmoid(const float* x, float* y, int64_t n, void* stream) {
+  DDSP_REQUIRE(x && y, DDSP_B200_E_INVALID, "sigmoid: null pointer");
+  DDSP_REQUIRE(n >= 0, DDSP_B200_E_INVALID, "sigmoid: n < 0");
+  if (n == 0) return 0;
+  sigmoid_kernel<<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>(x, y, n);
+  DDSP_CHECK_LAUNCH("sigmoid");
   return 0;
 }
 

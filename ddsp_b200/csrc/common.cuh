@@ -61,6 +61,13 @@ __device__ __forceinline__ float exp_sigmoid_f(float x) {
   return fmaf(2.0f, ex2_approx(-kLn10 * l), 1e-7f);
 }
 
+// tf.nn.sigmoid (ModDelay's default phase_scale_fn, effects.py:331-344):
+// 1 / (1 + e^-x) with e^-x on the SFU and a correctly rounded reciprocal; both
+// limits are exact (x -> -inf: 0, x -> +inf: 1).
+__device__ __forceinline__ float sigmoid_f(float x) {
+  return __frcp_rn(1.0f + ex2_approx(-x * 1.4426950408889634f));
+}
+
 // ---- Philox4x32-10 (Salmon et al., SC'11) ----------------------------------
 struct Philox4 {
   uint32_t x, y, z, w;

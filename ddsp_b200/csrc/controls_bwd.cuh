@@ -26,6 +26,15 @@ __device__ __forceinline__ float exp_sigmoid_grad(float x, float* y_out) {
   return core * kLn10 * one_minus_sig;
 }
 
+// sigmoid_f and its derivative s (1 - s), taken as t s^2 (t = e^-x) for x >= 0
+// where 1 - s would cancel.
+__device__ __forceinline__ float sigmoid_grad(float x, float* y_out) {
+  const float t = ex2_approx(-x * 1.4426950408889634f);
+  const float s = __frcp_rn(1.0f + t);
+  *y_out = s;
+  return x < 0.f ? s * (1.0f - s) : t * s * s;
+}
+
 // One warp per (b, i) row.
 //   dha[k]   = g0[i,k] + g1[i-1,k] (i > 0) + g1[F-1,k] (i == F-1)      (backward.cuh)
 //   n        = e / sum(e), e = exp_sigmoid(hd_raw) on the live prefix (f0 k < sr/2)

@@ -395,10 +395,34 @@ wt_amp_grad(const float* __restrict__ gl, const float* __restrict__ amps,
   }
 }
 
+// ---- core.linear_lookup's interpolation rule ---------------------------------------
+// A table of W + 1 entries whose entry W is entry 0, read at position x = phase W
+// (in double): entries floor(x) and floor(x) + 1 weigh 1 - frac and frac, and an
+// entry outside [0, W] weighs zero - the reference's relu(1 - |phase - j/W| W).
+// The indices come back in [0, W) (entry W as 0, an entry outside the table as 0
+// with ok = false), so both are always readable.  wt_linear_lookup and the
+// variable-length delay (mod_delay.cuh) both read their tables through this.
+struct LookupTaps {
+  int j0, j1;          // entry indices in [0, W)
+  bool ok0, ok1;       // inside [0, W]: weights 1 - fr and fr, else zero
+  double fr;
+};
+
+__device__ __forceinline__ LookupTaps lookup_taps(double x, int W) {
+  LookupTaps t;
+  const double fl = floor(x);
+  t.fr = x - fl;
+  t.ok0 = fl >= 0.0 && fl <= (double)W;
+  t.ok1 = fl + 1.0 >= 0.0 && fl + 1.0 <= (double)W;
+  const int j0 = t.ok0 ? (int)fl : 0;
+  const int j1 = t.ok1 ? (int)(fl + 1.0) : 0;
+  t.j0 = j0 == W ? 0 : j0;
+  t.j1 = j1 == W ? 0 : j1;
+  return t;
+}
+
 // ---- stand-alone core.linear_lookup ----------------------------------------------
-// phase [B, N] (any real value), tables [B, W] (static) or [B, N, W].  Entry W is
-// entry 0; x = phase W in double, weights 1 - frac / frac on floor(x) / floor(x) + 1,
-// entries outside [0, W] weigh zero (the reference's relu(1 - |phase - j/W| W)).
+// phase [B, N] (any real value), tables [B, W] (static) or [B, N, W].
 __global__ void __launch_bounds__(256)
 wt_linear_lookup(const float* __restrict__ phase, const float* __restrict__ tables,
                  float* __restrict__ out, int B, int N, int W, int per_sample) {
@@ -407,18 +431,10 @@ wt_linear_lookup(const float* __restrict__ phase, const float* __restrict__ tabl
        idx += (long long)gridDim.x * blockDim.x) {
     const long long b = idx / N;
     const float* T = tables + (per_sample ? (size_t)idx * W : (size_t)b * W);
-    const double x = (double)phase[idx] * (double)W;
-    const double fl = floor(x);
-    const double fr = x - fl;
+    const LookupTaps t = lookup_taps((double)phase[idx] * (double)W, W);
     double acc = 0.0;
-    if (fl >= 0.0 && fl <= (double)W) {
-      const int j = (int)fl;
-      acc += (1.0 - fr) * (double)T[j == W ? 0 : j];
-    }
-    if (fl + 1.0 >= 0.0 && fl + 1.0 <= (double)W) {
-      const int j = (int)(fl + 1.0);
-      acc += fr * (double)T[j == W ? 0 : j];
-    }
+    if (t.ok0) acc += (1.0 - t.fr) * (double)T[t.j0];
+    if (t.ok1) acc += t.fr * (double)T[t.j1];
     out[idx] = (float)acc;
   }
 }

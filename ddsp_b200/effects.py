@@ -1,14 +1,16 @@
 """Effects processors that consume the decoder's audio: `Reverb`,
-`FilteredNoiseReverb` and `FIRFilter` with the reference's constructors and
-semantics (`ddsp/effects.py:28-117, 202-278, 283-325`; SURVEY 8f-3; the next
-node after `Add` in `solo_instrument.gin:26-40`).
+`FilteredNoiseReverb`, `FIRFilter` and `ModDelay` with the reference's
+constructors and semantics (`ddsp/effects.py:28-117, 202-278, 283-393`; SURVEY
+8f-3; the next node after `Add` in `solo_instrument.gin:26-40`).
 
 `Reverb` is a long linear time-invariant convolution (48000-tap impulse
 response): `core.fft_convolve` routes one impulse response of 2048 taps and more
 per item to the hand-written partitioned overlap-save convolution
 (csrc/longconv.cuh); `FilteredNoiseReverb` draws that impulse response from a
 `FilteredNoise` synthesizer; `FIRFilter` is the time-varying filter of
-`FilteredNoise` applied to given audio and runs on the IR + FIR kernels."""
+`FilteredNoise` applied to given audio and runs on the IR + FIR kernels.
+`ModDelay` (chorus, flanger, vibrato) reads two taps of the audio's own history
+per sample in one kernel (csrc/mod_delay.cuh)."""
 import torch
 
 from ddsp_b200 import core
@@ -140,3 +142,66 @@ class FIRFilter(processors.Processor):
 
   def get_signal(self, audio, magnitudes):
     return core.frequency_filter(audio, magnitudes, window_size=self.window_size)
+
+
+class ModDelay(processors.Processor):
+  """Modulated delay times used in chorus, flanger, and vibrato effects
+  (effects.py:328-393).
+
+  gain and phase are audio-rate controls, [batch, n_samples, 1] or
+  [batch, n_samples].  get_signal is one kernel (`ddsp_b200_mod_delay_forward`):
+  the reference's [batch, n_samples, max_length] frames never exist.  Called for
+  the signal only with the default scale functions (core.exp_sigmoid for the gain,
+  core.sigmoid for the phase), the processor runs get_controls inside that kernel
+  (one launch from raw network outputs, bit-identical to the two steps).  Training
+  goes through autograd.mod_delay_train."""
+
+  def __init__(self,
+               center_ms=15.0,
+               depth_ms=10.0,
+               sample_rate=16000,
+               gain_scale_fn=core.exp_sigmoid,
+               phase_scale_fn=core.sigmoid,
+               add_dry=True,
+               name='mod_delay'):
+    super().__init__(name=name)
+    self.center_ms = center_ms
+    self.depth_ms = depth_ms
+    self.sample_rate = sample_rate
+    self.gain_scale_fn = gain_scale_fn
+    self.phase_scale_fn = phase_scale_fn
+    self.add_dry = add_dry
+
+  def delay_map(self):
+    """effects.py:381-386 in Python floats: (max_length, depth_phase,
+    center_phase); max_length truncates, as the reference's int() does."""
+    max_delay_ms = self.center_ms + self.depth_ms
+    max_length_samples = int(self.sample_rate / 1000.0 * max_delay_ms)
+    depth_phase = self.depth_ms / max_delay_ms
+    center_phase = self.center_ms / max_delay_ms
+    return max_length_samples, depth_phase, center_phase
+
+  def call(self, audio, gain, phase, return_outputs_dict=False, **kwargs):
+    for k in ['training', 'mask']:
+      kwargs.pop(k, None)
+    if (not return_outputs_dict and not kwargs and
+        self.gain_scale_fn is core.exp_sigmoid and self.phase_scale_fn is core.sigmoid):
+      max_length, depth_phase, center_phase = self.delay_map()
+      return core.mod_delay(audio, gain, phase, max_length, depth_phase, center_phase,
+                            add_dry=self.add_dry, scale=True)
+    return super().call(audio, gain, phase, return_outputs_dict=return_outputs_dict,
+                        **kwargs)
+
+  def get_controls(self, audio, gain, phase):
+    """effects.py:346-365."""
+    if self.gain_scale_fn is not None:
+      gain = self.gain_scale_fn(core.torch_float32(gain))
+    if self.phase_scale_fn is not None:
+      phase = self.phase_scale_fn(core.torch_float32(phase))
+    return {'audio': audio, 'gain': gain, 'phase': phase}
+
+  def get_signal(self, audio, gain, phase):
+    """effects.py:367-393."""
+    max_length, depth_phase, center_phase = self.delay_map()
+    return core.mod_delay(audio, gain, phase, max_length, depth_phase, center_phase,
+                          add_dry=self.add_dry, scale=False)

@@ -335,6 +335,34 @@ int ddsp_b200_wavetable_backward(const float* f0_hz, const float* amps,
 int ddsp_b200_linear_lookup(const float* phase, const float* tables, float* out, int B,
                             int N, int W, int per_sample, void* stream);
 
+/* Modulated delay: core.variable_length_delay / effects.ModDelay.get_signal
+ * (core.py:1285-1313, effects.py:328-393) in one pass over the audio.
+ * audio, phase [B,N], gain [B,N] or NULL (gain 1), L = max_length >= 1.  Sample n
+ * reads the entries e_k = audio[n-k] (0 <= k < L, zero before the start) and
+ * e_L = e_0 with linear_lookup's rule at position (phase*phase_scale +
+ * phase_offset)*L (double), times gain, + audio[n] when add_dry.
+ * variable_length_delay is phase_scale 1, phase_offset 0, no gain, no add_dry.
+ * scale != 0: gain and phase are raw network outputs and exp_sigmoid / sigmoid
+ * (ModDelay.get_controls' defaults) are applied inside the kernel, with the same
+ * device functions as ddsp_b200_noise_controls and ddsp_b200_sigmoid.
+ * backward: grad_out [B,N] -> d_audio [B,N], d_gain [B,N] (when gain), d_phase
+ * [B,N] (w.r.t. the raw inputs when scale != 0).  d_audio is summed in 64-bit
+ * fixed point with integer atomics: bit-reproducible, no float atomics.
+ * workspace: ddsp_b200_mod_delay_workspace(B,N,L) bytes (backward only). */
+size_t ddsp_b200_mod_delay_workspace(int B, int N, int L);
+int ddsp_b200_mod_delay_forward(const float* audio, const float* gain, const float* phase,
+                                float* out, int B, int N, int L, double phase_scale,
+                                double phase_offset, int scale, int add_dry,
+                                void* stream);
+int ddsp_b200_mod_delay_backward(const float* audio, const float* gain, const float* phase,
+                                 const float* grad_out, float* d_audio, float* d_gain,
+                                 float* d_phase, int B, int N, int L, double phase_scale,
+                                 double phase_offset, int scale, int add_dry,
+                                 void* workspace, size_t workspace_bytes, void* stream);
+/* tf.nn.sigmoid elementwise (core.sigmoid, ModDelay's default phase_scale_fn),
+ * n elements. */
+int ddsp_b200_sigmoid(const float* x, float* y, int64_t n, void* stream);
+
 /* core.resample / core.upsample_with_windows (core.py:573-714) stand-alone:
  * in [B,F,C] -> out [B,N,C].  method: 0 'window', 1 'linear', 2 'nearest',
  * 3 'cubic' (tf.compat.v1 bicubic, Keys A = -0.75).  add_endpoint as in the
